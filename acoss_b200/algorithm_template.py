@@ -52,6 +52,24 @@ def _load_feature_file(path):
         return out
 
 
+def _zeroed_memmap(path, shape):
+    """What ``np.memmap(path, mode="w+")`` gives (a zero float32 matrix backed by ``path``), without its window in
+    which the file is 0 bytes long: ranks that construct on the same cache prefix at once would otherwise fail to
+    map a file another rank has just truncated."""
+    nbytes = int(np.prod(shape)) * 4
+    fd = os.open(path, os.O_RDWR | os.O_CREAT, 0o666)
+    try:
+        size = os.fstat(fd).st_size
+        if size != nbytes:
+            os.ftruncate(fd, nbytes)
+    finally:
+        os.close(fd)
+    mm = np.memmap(path, mode="r+", dtype="float32", shape=shape)
+    if size:                                                 # a file that existed keeps old scores: clear them
+        mm[:] = 0
+    return mm
+
+
 class CoverAlgorithm(object):
     """
     Attributes
@@ -76,8 +94,7 @@ class CoverAlgorithm(object):
         os.makedirs(cachedir, exist_ok=True)                  # (several ranks of one box may construct at once)
         self.Ds = {}
         for s in similarity_types:
-            self.Ds[s] = np.memmap("%s_%s_dmat" % (self.get_cacheprefix(), s), shape=(self.N, self.N),
-                                   mode="w+", dtype="float32")
+            self.Ds[s] = _zeroed_memmap("%s_%s_dmat" % (self.get_cacheprefix(), s), (self.N, self.N))
         print("Initialized %s algorithm on %i songs in dataset %s" % (name, self.N, shortname))
 
     def get_cacheprefix(self):

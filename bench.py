@@ -28,13 +28,17 @@ Output: ONE JSON line on rank 0 (contract in the task statement), with
                oracle sample (DESIGN.md §4.5); `--no-earlyfusion` skips it
 `--impl reference` times that CPU port alone (the reference's essentia path cannot be installed:
 DESIGN.md §5) on the same config/metric/unit.
+`--dump-outputs DIR` writes the scores of the last timed step to DIR/scores.npy (float32), so that two builds run
+with the same arguments, hence on the same pairs, can be compared output for output.
 """
 import argparse
 import contextlib
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -42,6 +46,8 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True                                 # the tree bench.py runs from may be read-only
+DUMP_LIMIT = 64 << 20                                          # bytes written by --dump-outputs
 
 # Per-pair constants of the dominant kernel (the emit sweep) measured by the committed `ncu --set full` capture of
 # THIS build: DRAM bytes (dram__bytes_read.sum + dram__bytes_write.sum) and executed warp instructions
@@ -220,6 +226,15 @@ def c4s_leg(device):
             "fallback_pairs": st["fallback_pairs"], "parity_on_sample": bool(np.array_equal(got[sel], want))}
 
 
+def dump_outputs(dirname, scores):
+    """Scores of the last timed step as DIR/scores.npy; above DUMP_LIMIT a fixed, seeded sample of them."""
+    scores = np.asarray(scores, dtype=np.float32).reshape(-1)
+    if scores.nbytes > DUMP_LIMIT:
+        scores = scores[np.sort(np.random.default_rng(0).choice(scores.size, DUMP_LIMIT // 4, replace=False))]
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "scores.npy"), scores)
+
+
 def run_reference(args, rank, world):
     """--impl reference: the CPU port of the reference path, all host threads, bounded steps."""
     if rank != 0:
@@ -238,9 +253,11 @@ def run_reference(args, rank, world):
     ncell = 0
     for _ in range(args.steps):
         idx = pairs[sel[k0:k0 + per_step]]; k0 += per_step
-        oc.pairs(frames, offs, idx, p, nthreads=cores)
+        scores = oc.pairs(frames, offs, idx, p, nthreads=cores)
         ncell += algorithmic_bytes(lens, idx)[0]
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, scores)
     val = args.steps * per_step / dt
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt / args.steps * 1e3,
@@ -266,7 +283,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-earlyfusion", action="store_true", help="skip the secondary EarlyFusion leg")
     ap.add_argument("--crp-path", default="auto", choices=["auto", "exact"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the scores of the last timed step to DIR/scores.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -324,21 +344,26 @@ def main():
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    barrier()
-    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    launches = 0
-    with torch.cuda.stream(stream):
-        ev0.record(stream)
-        for k in range(args.warmup, total_steps):
-            step(k)
-            launches += eng.last_stats()["launches"]
-        if world > 1:
-            dist.all_gather_into_tensor(gathered, d_scores)      # NCCL gather of the per-rank score tiles
-        ev1.record(stream)
-    eng.sync()
-    barrier()
+    try:
+        barrier()
+        ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        launches = 0
+        with torch.cuda.stream(stream):
+            ev0.record(stream)
+            for k in range(args.warmup, total_steps):
+                step(k)
+                launches += eng.last_stats()["launches"]
+            if world > 1:
+                dist.all_gather_into_tensor(gathered, d_scores)      # NCCL gather of the per-rank score tiles
+            ev1.record(stream)
+        eng.sync()
+        barrier()
+    finally:
+        clocks = sampler.stop() if rank == 0 else None           # the sampler process must not outlive a failed run
     ms = ev0.elapsed_time(ev1)
-    clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        last = slice((total_steps - 1) * P, total_steps * P)
+        dump_outputs(args.dump_outputs, (gathered.view(world, need)[:, last] if world > 1 else d_scores[last]).cpu().numpy())
     stage = eng.stage_ms()
     kernel_ms_timed = eng.kernel_ms()
     k2_debug = eng.debug_counters()                            # of the last timed step
@@ -370,10 +395,10 @@ def main():
     # N x N matrix and its symmetrisation; then the reference's tail on rank 0 (normalize_by_length, getEvalStatistics)
     from acoss_b200.distributed import all_pairwise_distributed
     feats = [dict(hpcp=t_, label=str(l)) for t_, l in zip(tracks, labels)]
-    cache = os.path.join("/tmp", "acoss_bench_cache_%d" % rank)
+    workdir = tempfile.mkdtemp(prefix="acoss_bench_")          # score memmap and results csv of the plugin
     with contextlib.redirect_stdout(sys.stderr):               # keep stdout to the one JSON line
         alg = Serra09(None, None, features=feats, downsample_fac=1, shortname="bench%d" % rank, device=local,
-                      cachedir=cache, engine=eng, tile_pairs=P)
+                      cachedir=os.path.join(workdir, "cache"), engine=eng, tile_pairs=P)
     alg._resident = True                                       # tracks already resident in this engine
     alg.crp_path = params.crp_path
     alg.similarity(pairs[:4096].astype(np.int64))              # warm-up of the host path (pinned staging, allocations)
@@ -390,18 +415,15 @@ def main():
     e2e_val = len(pairs) / e2e_s
     tail = None
     if rank == 0:
-        with contextlib.redirect_stdout(sys.stderr):
+        with contextlib.redirect_stdout(sys.stderr), contextlib.chdir(workdir):   # results csv goes to the CWD
             tt0 = time.perf_counter()
             alg.normalize_by_length()
             tt1 = time.perf_counter()
             MR, MRR, MDR, MAP, tops = alg.getEvalStatistics("main")
             tt2 = time.perf_counter()
         tail = {"normalize_by_length_s": tt1 - tt0, "getEvalStatistics_s": tt2 - tt1, "MAP": float(MAP), "MR1": float(MR)}
-        try:
-            os.remove("results_bench0_Serra09.csv")
-        except OSError:
-            pass
     alg.cleanup_memmap()
+    shutil.rmtree(workdir, ignore_errors=True)
 
     # ---- roofline of the dominant kernel (the emit sweep, which writes the bit-packed CRP) ---------------------------
     k2_ms = stage["k2_crp"]

@@ -1,15 +1,15 @@
 """The drop-in boundary under the reference's OWN classes (VERDICT r1, "prove the boundary against the real class").
 
-Where /root/reference exists (the GPU-less build container): the unmodified ``acoss.algorithms.rqa_serra09.Serra09``
-(on its unmodified ``CoverAlgorithm`` base, imported through the SURVEY App. C shims) is subclassed by the
-INTEGRATION.md section B binding (``acoss_b200.integration.bind_serra09``) and runs the ``coverid.benchmark`` sequence
-(``/root/reference/acoss/coverid.py:57-70``) with the reference's own ``all_pairwise`` / ``normalize_by_length`` /
-``getEvalStatistics``.  No GPU here, so the binding talks to a CPU stand-in of the same C ABI backed by the oracle
-(``oracle/abi_stub.c``, test infrastructure).  The resulting score matrix and metrics are the committed golden
+With ``ACOSS_REFERENCE`` naming a checkout of the original acoss (github.com/furkanyesiler/acoss): the unmodified
+``acoss.algorithms.rqa_serra09.Serra09`` (on its unmodified ``CoverAlgorithm`` base, imported through the SURVEY
+App. C shims) is subclassed by the INTEGRATION.md section B binding (``acoss_b200.integration.bind_serra09``) and runs
+the ``coverid.benchmark`` sequence (``acoss/coverid.py:57-70``) with the reference's own ``all_pairwise`` /
+``normalize_by_length`` / ``getEvalStatistics``.  The binding talks to a CPU stand-in of the same C ABI backed by the
+oracle (``oracle/abi_stub.c``, test infrastructure).  The resulting score matrix and metrics are the committed golden
 ``tests/golden/refclass_tiny_golden.npz``.
 
-On the GPU box (no reference): ``acoss_b200.serra09.Serra09`` and the same binding on this package's mirror base
-class, both on the real ``libacoss_b200.so``, must reproduce that golden bit for bit."""
+Without the reference, the same binding on this package's mirror base class must reproduce that golden bit for bit:
+on the CPU stand-in, and on the real ``libacoss_b200.so`` together with ``acoss_b200.serra09.Serra09``."""
 import ctypes as C
 import os
 import sys
@@ -19,7 +19,7 @@ import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+REF = os.environ.get("ACOSS_REFERENCE", "")                # checkout of the original acoss (optional)
 GOLDEN = os.path.join(ROOT, "tests", "golden", "refclass_tiny_golden.npz")
 TOPS = [1, 10]
 
@@ -97,7 +97,7 @@ def shimmed_reference():
     sys.path[:] = path
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="/root/reference is not present (GPU box): the committed golden stands in")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="ACOSS_REFERENCE names no checkout of acoss: the committed golden stands in")
 def test_binding_under_the_reference_classes(tmp_path, monkeypatch, shimmed_reference):
     monkeypatch.chdir(tmp_path)                              # the reference writes cache/ and results_*.csv into the CWD
     from acoss.algorithms.algorithm_template import CoverAlgorithm as RefCoverAlgorithm
@@ -141,6 +141,43 @@ def _run_sequence(alg):
     return raw, Dn, np.array([MR, MRR, MDR, MAP] + list(tops), dtype=np.float64)
 
 
+def _serial_serra09():
+    from acoss_b200.serra09 import Serra09
+
+    class SerialSerra09(Serra09):                            # the reference's serial driver: one pair per call
+        def all_pairwise(self, parallel=0, n_cores=12, symmetric=False, precomputed=False):
+            for i, j in self._pair_array(symmetric):
+                self.similarity(np.array([[i, j]]))
+            if symmetric:
+                for key in self.Ds:
+                    self.Ds[key] += self.Ds[key].T
+    return SerialSerra09
+
+
+def _bound_sequence(lib=None):
+    """The INTEGRATION.md section B binding on the mirror base class, one pair per similarity() call."""
+    from acoss_b200.algorithm_template import CoverAlgorithm
+    from acoss_b200.integration import bind_serra09
+    Bound = bind_serra09(_serial_serra09(), lib=lib)
+    assert issubclass(Bound, CoverAlgorithm)
+    tracks, labels = _tiny()
+    feats = [dict(hpcp=t, label=l) for t, l in zip(tracks, labels)]
+    alg = Bound(None, None, features=feats, downsample_fac=1, shortname="tinyb")
+    raw, Dn, metrics = _run_sequence(alg)
+    alg.release()
+    return raw, Dn, metrics
+
+
+def test_binding_on_the_cpu_abi_stub_reproduces_the_reference_class_golden(tmp_path, monkeypatch):
+    """The binding on the CPU stand-in of the C ABI == the golden produced under the reference's own classes."""
+    monkeypatch.chdir(tmp_path)
+    from oracle import build as obuild
+    raw, Dn, metrics = _bound_sequence(C.CDLL(obuild.build_stub()))
+    g = np.load(GOLDEN)
+    assert np.array_equal(g["raw"], raw) and np.array_equal(g["normalized"], Dn)
+    assert np.array_equal(g["metrics"], metrics)
+
+
 @pytest.mark.gpu
 def test_gpu_plugin_reproduces_the_reference_class_golden(tmp_path, monkeypatch):
     """acoss_b200.serra09.Serra09 (batched GPU path) == the golden produced under the reference's own classes."""
@@ -161,24 +198,7 @@ def test_gpu_binding_reproduces_the_reference_class_golden(tmp_path, monkeypatch
     """The INTEGRATION.md section B binding on the real libacoss_b200.so, one pair per similarity() call through the
     base class's serial all_pairwise (the mirror base here; the reference's base in the CPU test above)."""
     monkeypatch.chdir(tmp_path)
-    from acoss_b200.integration import bind_serra09
-    from acoss_b200.serra09 import Serra09
-    from acoss_b200.algorithm_template import CoverAlgorithm
-
-    class SerialSerra09(Serra09):                            # the reference's serial driver: one pair per call
-        def all_pairwise(self, parallel=0, n_cores=12, symmetric=False, precomputed=False):
-            for i, j in self._pair_array(symmetric):
-                self.similarity(np.array([[i, j]]))
-            if symmetric:
-                for key in self.Ds:
-                    self.Ds[key] += self.Ds[key].T
-    Bound = bind_serra09(SerialSerra09)
-    assert issubclass(Bound, CoverAlgorithm)
-    tracks, labels = _tiny()
-    feats = [dict(hpcp=t, label=l) for t, l in zip(tracks, labels)]
-    alg = Bound(None, None, features=feats, downsample_fac=1, shortname="tinyb")
-    raw, Dn, metrics = _run_sequence(alg)
-    alg.release()
+    raw, Dn, metrics = _bound_sequence()
     g = np.load(GOLDEN)
     assert np.array_equal(g["raw"], raw) and np.array_equal(g["normalized"], Dn)
     assert np.array_equal(g["metrics"], metrics)
