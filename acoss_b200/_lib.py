@@ -9,8 +9,7 @@ import ctypes as C
 import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-# ACOSS_B200_LIB: alternative build of the same ABI (A/B timing of kernel variants)
-LIB_PATH = os.environ.get("ACOSS_B200_LIB") or os.path.join(HERE, "csrc", "libacoss_b200.so")
+LIB_PATH = os.path.join(HERE, "csrc", "libacoss_b200.so")
 
 OK, E_INVALID, E_CUDA, E_TOO_SHORT, E_NAN, E_NONBINARY, E_NOMEM = 0, -1, -2, -3, -4, -5, -6
 ALIGN_QMAX, ALIGN_SW, ALIGN_DMAX, ALIGN_DMAX_PLAIN = 0, 1, 2, 3

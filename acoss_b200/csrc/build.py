@@ -7,10 +7,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 SOURCES = ["api.cu", "k0_onramp.cu", "k1_oti.cu", "k2_exact.cu", "k2_fast.cu", "k3_dp.cu", "k4_knn.cu", "k5_earlyfusion.cu"]
 HEADERS = ["common.cuh", "k2_fast.cuh", "k2_tc.inl", "../../include/acoss_b200.h"]
 OUT = os.path.join(HERE, "libacoss_b200.so")
-import os as _os
-EXTRA = _os.environ.get("ACOSS_NVCC_EXTRA", "").split()
-NVCC_FLAGS = EXTRA + ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
-              "-Xcompiler", "-fPIC", "--use_fast_math=false" if False else "-Xcompiler", "-O2"]
+NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
+              "-Xcompiler", "-fPIC", "-Xcompiler", "-O2"]
 
 
 def needs_build() -> bool:

@@ -6,7 +6,7 @@
 // reference-order arithmetic of k2_exact.cu.  The three sweeps over the cell matrix (row thresholds, column
 // thresholds, emit) exist twice and launch_k2_fast picks per call: on the tensor cores (k2_tc.inl: the stacked
 // 108-term inner product as an exact integer GEMM, tcgen05.mma kind::i8 over byte-limb planes, items read from
-// tensor memory) for lines of K2_TC_MIN_WINDOWS windows or more, and as FFMA2 chains on the CUDA cores (this file)
+// tensor memory) for lines of TC_MIN_WINDOWS windows or more, and as FFMA2 chains on the CUDA cores (this file)
 // for short lines and for features that cannot be quantised inside the error budget.  Everything around the sweeps
 // (prep, sampler, selection, candidate lists, exact thresholds, bit patch) is shared.  Structure of the FFMA2 form:
 //
@@ -40,10 +40,7 @@ constexpr int M9 = 9;               // frameStackSize handled by this path
 constexpr int HALO = M9 - 1;        // owned columns a strip recomputes (8)
 constexpr int NBIN = 64;            // histogram bins per level (+ one underflow and one overflow row)
 constexpr int SBIN = 256;           // bins of the per-line sample histogram (select kernel)
-#ifndef K2_EPS
-#define K2_EPS 128
-#endif
-constexpr int EPS = K2_EPS;            // bound on |z - exact item| in fixed-point units (DESIGN.md §4.2)
+constexpr int EPS = 128;            // bound on |z - exact item| in fixed-point units (DESIGN.md §4.2)
 constexpr int CAND_CAP = 128;       // candidates per row / column
 constexpr int BRACKET_TARGET = 96;  // a bracket holding more cells than this is split by another histogram level
 constexpr int WPC = 4;              // warps per CTA in the sweep kernels
@@ -51,24 +48,9 @@ constexpr int TC_N = 64;            // streamed windows per tensor-sweep block (
 constexpr int TC_PAD = 2 * TC_N;    // padding of per-window arrays and byte planes read in whole blocks
 constexpr int TC_HUGE = 0x20000000; // norm of a padding window: its items land above every bracket
 constexpr int RCV = 4;              // owned frames per lane (register columns) in the sweep kernels
-#ifndef K2_FFMA2
-#define K2_FFMA2 1                  // 1: packed fma.rn.f32x2 dot products (FFMA2); 0: the same chains as scalar FFMA
-#endif
-#ifndef K2_SPLIT
-#define K2_SPLIT 1                  // FMA chains per (even, odd) half of a dot product: 1 = six steps each, 2 = two chains of three
-#endif
-#ifndef K2_HRC
-#define K2_HRC 4                    // register columns per lane of the histogram sweeps
-#endif
-#ifndef K2_HMINB
-#define K2_HMINB K2_MINB            // CTAs per SM the histogram sweeps are compiled for
-#endif
-#ifndef K2_TC_MIN_WINDOWS
-#define K2_TC_MIN_WINDOWS 400        // longer side of the matrix from which the tensor sweeps (k2_tc.inl) replace the FFMA2 sweeps
-#endif
-#ifndef K2_MINB
-#define K2_MINB 3                   // CTAs per SM the sweep kernels are compiled for (register cap 168 at 3, 255 at 2)
-#endif
+constexpr int HRC = 4;              // register columns per lane of the histogram sweeps
+constexpr int MINB = 3;             // CTAs per SM the sweep kernels are compiled for (register cap 168 at 3, 255 at 2)
+constexpr int TC_MIN_WINDOWS = 400; // longer side of the matrix from which the tensor sweeps (k2_tc.inl) replace the FFMA2 sweeps
 
 struct PairHdr {                    // per-slot header written by fast_prep_kernel
     int32_t nq, nr, Mx, Nx;         // frames and stacked windows of query / reference
@@ -136,8 +118,6 @@ FastLayout make_layout(const SlotGeom &g, int max_frames) {
         // short lines: keep at least 32 samples per line (a bracket from fewer samples is too wide to help;
         // measured at 500 frames: S = 16 or 8 give +30 % pairs/s over S = 32, at 2k frames S = 32 is best)
         while (L.slog > 2 && (Lmax >> L.slog) < 32) --L.slog;
-        static const char *force = getenv("ACOSS_K2_SLOG");    // tuning switch
-        if (force && force[0] >= '2' && force[0] <= '5') L.slog = force[0] - '0';
     }
     L.nst_r = ((g.max_cols - 1) >> L.slog) + 1;
     L.nst_c = ((g.max_rows - 1) >> L.slog) + 1;
@@ -187,19 +167,18 @@ __device__ __forceinline__ u64 ffma2(u64 a, u64 b, u64 c) {
     return d;
 }
 // raw bits of the two half chains, summed (= quantised 2<x, y> + 2 * bits(magic)); x, y: 12 floats each
-constexpr int NMAGIC = 2 * K2_SPLIT;                // magic offsets inside one quantised dot product
+constexpr int NMAGIC = 2;                           // magic offsets inside one quantised dot product
 __device__ __forceinline__ int dot_fx(const float (&x)[NBINS], const float (&y)[NBINS], float magic) {
+    float acc[2] = {magic, magic};                  // even bins, odd bins
+#pragma unroll
+    for (int b = 0; b < NBINS; b += 2)
+#pragma unroll
+        for (int h = 0; h < 2; ++h) acc[h] = __fmaf_rn(x[b + h], y[b + h], acc[h]);
+    // summed in a loop, not as one expression: the compiler then keeps (even + odd) - magic offsets in the callers
+    // instead of reassociating it (as one expression the sampler measured 5 % slower on a B200)
     int r = 0;
 #pragma unroll
-    for (int c = 0; c < K2_SPLIT; ++c) {           // bins [c * 12 / SPLIT, (c + 1) * 12 / SPLIT): one (even, odd) chain pair
-        float ae = magic, ao = magic;
-#pragma unroll
-        for (int b = c * (NBINS / K2_SPLIT); b < (c + 1) * (NBINS / K2_SPLIT); b += 2) {
-            ae = __fmaf_rn(x[b], y[b], ae);
-            ao = __fmaf_rn(x[b + 1], y[b + 1], ao);
-        }
-        r += __float_as_int(ae) + __float_as_int(ao);
-    }
+    for (int h = 0; h < 2; ++h) r += __float_as_int(acc[h]);
     return r;
 }
 __device__ __forceinline__ void load_frame(const float *__restrict__ p, float (&x)[NBINS], float scale) {
@@ -495,51 +474,14 @@ struct Sweep {
 
     // frame-level dot products of one streamed frame (six (even, odd) pairs) with the lane's RC owned frames
     __device__ __forceinline__ void dot(const ulonglong2 &x0, const ulonglong2 &x1, const ulonglong2 &x2, int (&eb)[RC]) const {
-#if K2_FFMA2
         const u64 xs[6] = {x0.x, x0.y, x1.x, x1.y, x2.x, x2.y};
-        u64 acc[K2_SPLIT][RC];
-        constexpr int PER = 6 / K2_SPLIT;             // packed steps per chain
+        u64 acc[RC];
 #pragma unroll
-        for (int t = 0; t < PER; ++t)
+        for (int t = 0; t < 6; ++t)
 #pragma unroll
-            for (int c = 0; c < K2_SPLIT; ++c)
+            for (int k = 0; k < RC; ++k) acc[k] = ffma2(xs[t], y[k][t], t == 0 ? magic2 : acc[k]);
 #pragma unroll
-                for (int k = 0; k < RC; ++k)
-                    acc[c][k] = ffma2(xs[c * PER + t], y[k][c * PER + t], t == 0 ? magic2 : acc[c][k]);
-#pragma unroll
-        for (int k = 0; k < RC; ++k) {
-            int e = 0;
-#pragma unroll
-            for (int c = 0; c < K2_SPLIT; ++c) e += (int)(unsigned)(acc[c][k] & 0xffffffffu) + (int)(unsigned)(acc[c][k] >> 32);
-            eb[k] = e;
-        }
-#else
-        // the same chains per column as scalar FFMA (bit-identical halves)
-        const u64 xs[6] = {x0.x, x0.y, x1.x, x1.y, x2.x, x2.y};
-        const float mg = __uint_as_float((unsigned)(magic2 & 0xffffffffu));
-        constexpr int PER = 6 / K2_SPLIT;
-        float ae[K2_SPLIT][RC], ao[K2_SPLIT][RC];
-#pragma unroll
-        for (int t = 0; t < PER; ++t)
-#pragma unroll
-            for (int c = 0; c < K2_SPLIT; ++c) {
-                const u64 xv = xs[c * PER + t];
-                const float xe = __uint_as_float((unsigned)(xv & 0xffffffffu)), xo = __uint_as_float((unsigned)(xv >> 32));
-#pragma unroll
-                for (int k = 0; k < RC; ++k) {
-                    const u64 yv = y[k][c * PER + t];
-                    ae[c][k] = __fmaf_rn(xe, __uint_as_float((unsigned)(yv & 0xffffffffu)), t == 0 ? mg : ae[c][k]);
-                    ao[c][k] = __fmaf_rn(xo, __uint_as_float((unsigned)(yv >> 32)), t == 0 ? mg : ao[c][k]);
-                }
-            }
-#pragma unroll
-        for (int k = 0; k < RC; ++k) {
-            int e = 0;
-#pragma unroll
-            for (int c = 0; c < K2_SPLIT; ++c) e += __float_as_int(ae[c][k]) + __float_as_int(ao[c][k]);
-            eb[k] = e;
-        }
-#endif
+        for (int k = 0; k < RC; ++k) eb[k] = (int)(unsigned)(acc[k] & 0xffffffffu) + (int)(unsigned)(acc[k] >> 32);
     }
 
     // slides the diagonal sums T by one row.  U = a % 9 (static ring slot).
@@ -747,7 +689,7 @@ constexpr int DENSE2_MIN_LIVE = 16;  // live lines a strip must hold for the sec
 // and the next level splits it).
 // ------------------------------------------------------------------------------------------------
 template <int RC, int ORIENT>
-__global__ void __launch_bounds__(32 * WPC, K2_HMINB) fast_hist_kernel(TrackSet ts, const int32_t *__restrict__ pairs,
+__global__ void __launch_bounds__(32 * WPC, MINB) fast_hist_kernel(TrackSet ts, const int32_t *__restrict__ pairs,
                                                              int64_t first, int n, FastLayout L,
                                                              char *__restrict__ scratch, int strips_max, float magic,
                                                              uint32_t *__restrict__ status, uint32_t *__restrict__ dbg,
@@ -1017,7 +959,7 @@ __device__ __forceinline__ unsigned transpose_nibbles(unsigned x, unsigned selA,
 }
 
 template <int RC>
-__global__ void __launch_bounds__(32 * WPC, K2_MINB) fast_emit_kernel(TrackSet ts, const int32_t *__restrict__ pairs,
+__global__ void __launch_bounds__(32 * WPC, MINB) fast_emit_kernel(TrackSet ts, const int32_t *__restrict__ pairs,
                                                              int64_t first, int n, FastLayout L,
                                                              char *__restrict__ scratch, int groups, float magic,
                                                              uint32_t *__restrict__ crp_all, int words,
@@ -1309,12 +1251,6 @@ __global__ void __launch_bounds__(256) fast_rank_kernel(int n, FastLayout L, cha
         cnt = (int)min(c, (unsigned)CAND_CAP);
     }
     if (sub == 0) { s_wn[grp][0] = 0; s_wn[grp][1] = 0; s_zsel[grp][0] = 0; s_zsel[grp][1] = 0; }
-#ifdef K2_DEBUG_CNT
-    if (sub == 0 && live) {                                   // candidate-count statistics: lines, sum, sum of squares / 64, max, > 64
-        atomicAdd(&dbg[26], 1u); atomicAdd(&dbg[27], (unsigned)cnt); atomicAdd(&dbg[28], (unsigned)(cnt * cnt) >> 6);
-        atomicMax(&dbg[29], (unsigned)cnt); if (cnt > 64) atomicAdd(&dbg[30], 1u);
-    }
-#endif
     for (int p = sub; p < cnt; p += 8) {
         s_z[grp][p] = candz[p];
         nbelow += cand[p] >> 15;
@@ -1580,18 +1516,17 @@ int launch_k2_fast(const TrackSet &ts, const int32_t *pairs, const int32_t *oti,
     auto tb = [&](int id) { if (timer) timer->begin(id); };
     auto te = [&](int id) { if (timer) timer->end(id); };
     tb(K2K_PREP);
-    // Sweeps: tensor cores from K2_TC_MIN_WINDOWS windows on the longer side (a CTA's fixed costs - TMEM allocation, operand
+    // Sweeps: tensor cores from TC_MIN_WINDOWS windows on the longer side (a CTA's fixed costs - TMEM allocation, operand
     // fill, histogram scan - weigh on short lines; measured against the FFMA2 sweeps: +17 % pairs/s at 2 000 frames, level at
     // 500), FFMA2 below and whenever the features cannot be quantised within the error budget.  ACOSS_K2_SWEEPS=tc|ffma forces one of them (A/B runs, parity tests of both).
     const char *sweeps_env = getenv("ACOSS_K2_SWEEPS");          // read per call: tests flip it inside one process
-    bool use_tc = ts.q_exp >= 0 && std::max(g.max_rows, g.max_cols) >= K2_TC_MIN_WINDOWS;
+    bool use_tc = ts.q_exp >= 0 && std::max(g.max_rows, g.max_cols) >= TC_MIN_WINDOWS;
     if (sweeps_env && sweeps_env[0] == 't') use_tc = ts.q_exp >= 0;
     if (sweeps_env && sweeps_env[0] == 'f') use_tc = false;
     const float q_scale = use_tc ? ldexpf(1.f, ts.q_exp) : 0.f;
     fast_prep_kernel<<<n, 256, 0, st>>>(ts, pairs, oti, first, L, base, qperc, p.integer_guard, fx_scale, q_scale);
     CUDA_TRY(cudaGetLastError());
     te(K2K_PREP);
-    constexpr int HRC = K2_HRC;
     const int outw = Sweep<RC>::OUTW, houtw = Sweep<HRC>::OUTW;
     const int strips_c = (g.max_cols + outw - 1) / outw;                  // emit strips
     const int hstrips_c = (g.max_cols + houtw - 1) / houtw, hstrips_r = (g.max_rows + houtw - 1) / houtw;
@@ -1611,8 +1546,7 @@ int launch_k2_fast(const TrackSet &ts, const int32_t *pairs, const int32_t *oti,
     const int lines = g.max_rows + g.max_cols;
     // first brackets from every S-th diagonal (sampler + per-line selection), then up to three histogram
     // levels per orientation; a level returns immediately for strips whose lines are all done
-    static const bool no_sample = getenv("ACOSS_K2_NO_SAMPLE") != nullptr;   // debugging: start from the whole item range
-    if (!no_sample) {
+    {
         const int nu_max = ((g.max_rows - 1) >> L.slog) + ((g.max_cols - 1) >> L.slog) + 1;
         const int ngrp = (nu_max + SKD - 1) / SKD, nblk = (g.max_rows + SPOS - 1) / SPOS;
         const int64_t warps = (int64_t)n * ngrp * nblk;
@@ -1716,7 +1650,7 @@ int launch_k2_fast(const TrackSet &ts, const int32_t *pairs, const int32_t *oti,
     te(K2K_BITS);
     // kernels launched above: prep, sample, select, sparse, emit, scatter, rank, exact, thr, bits + the histogram sweeps (one
     // launch per orientation on the tensor cores, two with the FFMA2 sweeps)
-    if (launches) *launches += (no_sample ? 8 : 10) + (use_tc ? 2 : 4);
+    if (launches) *launches += 10 + (use_tc ? 2 : 4);
     return ACOSS_OK;
 }
 

@@ -14,16 +14,9 @@
 // inputs; its float32 features make BLAS-order-dependent float32 CSMs — the float64 value is the
 // one every BLAS approximates, and it is what the pinned oracle computes).  These are genuine
 // GEMMs (K = 480 / 1000 / 1225) but float64 ones, so tcgen05 (no float64 kind) does not apply; the
-// float64 tensor path of sm_100a is the warp-level DMMA.  Three generations of the contraction live
-// here, selectable with ACOSS_EF_CSM=1|2|3 for A/B timing (profiles/r1_ef.md):
-//   1  ef_csm_kernel   DFMA, 8x4 register tiles, k-major shared tiles          13.7 TFLOP/s
-//   2  ef_csm2_kernel  DFMA, 8x8 register tiles, row-major cp.async tiles      19.6 TFLOP/s
-//   3  ef_csm3_kernel  DMMA m8n8k4, 2x2 warps of 32x32, cp.async (production)   30.4 TFLOP/s
-// The DFMA kernels add the k terms of a cell in ascending k, one fused multiply-add per term; the DMMA kernel
-// produces bit-identical matrices (tools/ef_cmp_generations.py on a B200: all four matrices of a 300-block pair equal
-// across the three generations), i.e. the instruction behaves as the same ascending-k FMA chain.
-#include <stdlib.h>
-
+// float64 tensor path of sm_100a is the warp-level DMMA (ef_csm3_kernel: m8n8k4, 2x2 warps of 32x32,
+// cp.async, 30.4 TFLOP/s).  It adds the k terms of a cell as an ascending-k FMA chain.  The two DFMA
+// generations it replaced are described, with their measurements, in DESIGN.md §4.5.
 #include <algorithm>
 
 #include "common.cuh"
@@ -123,136 +116,17 @@ int launch_ef_oti(const double *cmed, const int32_t *pairs, int n, int32_t *oti,
 }
 
 // ---------------------------------------------------------------------------------------------
-// CSM: one 64x64 tile of one pair per CTA
+// CSM: one 64x64 tile of one pair per CTA, on the float64 tensor path (DMMA, mma.sync.m8n8k4.f64 — tcgen05
+// has no float64 kind; on sm_100a the legacy warp-level MMA is the only float64 tensor instruction).  One
+// DMMA replaces 8 DFMA per lane and needs one A and one B double per lane: 2 x 2 warps of 32 x 32 (4 x 4
+// MMA tiles, 32 accumulator doubles per lane), 8 LDS.64 per 16 DMMA.  Shared tiles are row-major [row][k]
+// with a pitch of 20 doubles, so the 4 rows x 4 k a half-warp reads fall in 32 distinct banks.  Global ->
+// shared goes through cp.async (16 B chunks, two-stage ring, no staging registers).
 // ---------------------------------------------------------------------------------------------
 #define EF_BM 64
 #define EF_BN 64
 #define EF_BK 16
-#define EF_PITCH 66     // doubles per k-row of a shared tile (16-byte aligned rows, staggered banks)
-
-// MODE 0: sqrt(max(0, (|x|^2 + |y|^2) - 2 x.y)); MODE 1: 1 - xhat.yhat with the 12-bin groups of x rolled by oti
-template <int MODE>
-__global__ void __launch_bounds__(128) ef_csm_kernel(const double *__restrict__ feat, int dp, int d,
-                                                     const double *__restrict__ sq,
-                                                     const int64_t *__restrict__ offsets,
-                                                     const int32_t *__restrict__ pairs,
-                                                     const int32_t *__restrict__ oti_a,
-                                                     double *__restrict__ csm, int64_t slot_elems, int tiles_n) {
-    __shared__ __align__(16) double As[EF_BK][EF_PITCH];
-    __shared__ __align__(16) double Bs[EF_BK][EF_PITCH];
-    const int slot = blockIdx.y;
-    const int q = pairs[2 * slot], r = pairs[2 * slot + 1];
-    const int64_t oq = offsets[q], orr = offsets[r];
-    const int M = (int)(offsets[q + 1] - oq), N = (int)(offsets[r + 1] - orr);
-    const int m0 = (blockIdx.x / tiles_n) * EF_BM, n0 = (blockIdx.x % tiles_n) * EF_BN;
-    if (m0 >= M || n0 >= N) return;
-    const int tid = threadIdx.x;
-    // global -> register staging: thread = (tile row, 8 consecutive k)
-    const int lrow = tid & 63, kh = (tid >> 6) * 8;
-    const double *ga = feat + (oq + min(m0 + lrow, M - 1)) * (int64_t)dp;
-    const double *gb = feat + (orr + min(n0 + lrow, N - 1)) * (int64_t)dp;
-    int rot = 0;
-    if (MODE == 1) rot = oti_a[slot];
-    // register tile: rows 2rg + {0,1} + 16 s (s = 0..3), columns 2cg + {0,1} + 32 h (h = 0,1)
-    const int rg = tid >> 4, cg = tid & 15;
-    double acc[8][4];
-#pragma unroll
-    for (int i = 0; i < 8; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) acc[i][j] = 0.0;
-    double ra[8], rb[8];
-    auto fetch = [&](int k0) {
-        if (MODE == 1) {
-#pragma unroll
-            for (int e = 0; e < 8; ++e) {
-                const int k = k0 + kh + e;
-                int src = k;
-                if (k < d) {                                 // np.roll(X1, oti, axis=2): out[b] = in[(b - oti) mod 12]
-                    const int t = k / NBINS, b = k - t * NBINS;
-                    src = t * NBINS + rot_src(b, rot);
-                }
-                ra[e] = ga[src];
-            }
-        } else {
-#pragma unroll
-            for (int e = 0; e < 8; e += 2) {
-                const double2 v = *reinterpret_cast<const double2 *>(ga + k0 + kh + e);
-                ra[e] = v.x; ra[e + 1] = v.y;
-            }
-        }
-#pragma unroll
-        for (int e = 0; e < 8; e += 2) {
-            const double2 v = *reinterpret_cast<const double2 *>(gb + k0 + kh + e);
-            rb[e] = v.x; rb[e + 1] = v.y;
-        }
-    };
-    fetch(0);
-    for (int k0 = 0; k0 < dp; k0 += EF_BK) {
-        __syncthreads();
-#pragma unroll
-        for (int e = 0; e < 8; ++e) { As[kh + e][lrow] = ra[e]; Bs[kh + e][lrow] = rb[e]; }
-        __syncthreads();
-        if (k0 + EF_BK < dp) fetch(k0 + EF_BK);
-#pragma unroll
-        for (int kk = 0; kk < EF_BK; ++kk) {
-            double a[8], b[4];
-#pragma unroll
-            for (int s = 0; s < 4; ++s) {
-                const double2 v = *reinterpret_cast<const double2 *>(&As[kk][2 * rg + 16 * s]);
-                a[2 * s] = v.x; a[2 * s + 1] = v.y;
-            }
-#pragma unroll
-            for (int h = 0; h < 2; ++h) {
-                const double2 v = *reinterpret_cast<const double2 *>(&Bs[kk][2 * cg + 32 * h]);
-                b[2 * h] = v.x; b[2 * h + 1] = v.y;
-            }
-#pragma unroll
-            for (int i = 0; i < 8; ++i)
-#pragma unroll
-                for (int j = 0; j < 4; ++j) acc[i][j] = fma(a[i], b[j], acc[i][j]);
-        }
-    }
-    double *out = csm + (int64_t)slot * slot_elems;
-    double sy[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-        const int col = n0 + 2 * cg + (j & 1) + 32 * (j >> 1);
-        sy[j] = (MODE == 0 && col < N) ? sq[orr + col] : 0.0;
-    }
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-        const int row = m0 + 2 * rg + (i & 1) + 16 * (i >> 1);
-        if (row >= M) continue;
-        const double sx = (MODE == 0) ? sq[oq + row] : 0.0;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            const int col = n0 + 2 * cg + (j & 1) + 32 * (j >> 1);
-            if (col >= N) continue;
-            double v;
-            if (MODE == 0) {
-                double c2 = __dsub_rn(__dadd_rn(sx, sy[j]), __dmul_rn(2.0, acc[i][j]));
-                c2 = c2 < 0.0 ? 0.0 : c2;
-                v = sqrt(c2);
-            } else {
-                v = __dsub_rn(1.0, acc[i][j]);
-            }
-            out[(int64_t)row * N + col] = v;
-        }
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
-// CSM, second generation.  ncu on the kernel above (profiles/r1_ef_csm.md): the shared-memory pipe is the
-// limiter (l1tex throughput 91 %, FP64 pipe 45 %) — an LDS.128 is served per half-warp, 128 B per wavefront,
-// so the 2 x 16 thread layout pays 4 wavefronts per B fragment.  Here: 64-thread CTAs (2 warps), 8 x 8
-// accumulators per thread, warp = 4 row groups x 8 column groups, tiles kept ROW-major in shared memory
-// ([row][k], pitch 18 doubles) so that one LDS.128 delivers two consecutive k of a row and every half-warp
-// touches exactly 128 distinct bytes (B) or 32 (A): 32 wavefronts per 128 DFMA per warp, half the pipe.
-// Global -> shared goes through cp.async (16 B chunks, two-stage ring), no staging registers.  The k order
-// of every accumulator is unchanged (k ascending, one FMA per k), so the results are bit-identical to the
-// first-generation kernel's.
-// ---------------------------------------------------------------------------------------------
-#define EF2_LD 18
+#define EF3_LD 20
 #define EF2_MAXDP 2048   // widest (padded) chroma block the rolled-column map covers
 __device__ __forceinline__ void ef_cp_async16(void *smem, const void *g) {
     const unsigned sa = (unsigned)__cvta_generic_to_shared(smem);
@@ -263,134 +137,6 @@ __device__ __forceinline__ void ef_cp_async8(void *smem, const void *g) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n" ::"r"(sa), "l"(g) : "memory");
 }
 
-// 16 k of one 64 x 64 tile for one thread: acc[i][j] += A[row_i][k] * B[col_j][k], k ascending
-#ifdef ACOSS_EF_GENERATIONS   // superseded generation 2 (DFMA 8x8, cp.async): compiled only for tools/ef_cmp_generations.py
-template <bool FULL>
-__device__ __forceinline__ void ef_tile_fma(const double *Ap, const double *Bp, int jmax, double (&acc)[8][8]) {
-#pragma unroll
-    for (int k2 = 0; k2 < EF_BK; k2 += 2) {
-        double2 a[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) a[i] = *reinterpret_cast<const double2 *>(Ap + i * 4 * EF2_LD + k2);
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            if (!FULL && j >= jmax) break;                    // warp-uniform
-            const double2 b = *reinterpret_cast<const double2 *>(Bp + j * 8 * EF2_LD + k2);
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                acc[i][j] = fma(a[i].x, b.x, acc[i][j]);
-                acc[i][j] = fma(a[i].y, b.y, acc[i][j]);
-            }
-        }
-    }
-}
-
-template <int MODE>
-__global__ void __launch_bounds__(64) ef_csm2_kernel(const double *__restrict__ feat, int dp, int d,
-                                                     const double *__restrict__ sq,
-                                                     const int64_t *__restrict__ offsets,
-                                                     const int32_t *__restrict__ pairs,
-                                                     const int32_t *__restrict__ oti_a,
-                                                     double *__restrict__ csm, int64_t slot_elems, int tiles_n) {
-    __shared__ __align__(16) double As[2][EF_BM][EF2_LD];
-    __shared__ __align__(16) double Bs[2][EF_BN][EF2_LD];
-    __shared__ short kmap[MODE == 1 ? EF2_MAXDP : 1];
-    const int slot = blockIdx.y;
-    const int q = pairs[2 * slot], r = pairs[2 * slot + 1];
-    const int64_t oq = offsets[q], orr = offsets[r];
-    const int M = (int)(offsets[q + 1] - oq), N = (int)(offsets[r + 1] - orr);
-    const int m0 = (blockIdx.x / tiles_n) * EF_BM, n0 = (blockIdx.x % tiles_n) * EF_BN;
-    if (m0 >= M || n0 >= N) return;
-    const int tid = threadIdx.x;
-    const double *Abase = feat + oq * (int64_t)dp, *Bbase = feat + orr * (int64_t)dp;
-    if (MODE == 1) {                                          // np.roll(X1, oti, axis=2): out[b] = in[(b - oti) mod 12]
-        const int rot = oti_a[slot];
-        for (int k = tid; k < dp; k += 64) {
-            int src = k;
-            if (k < d) {
-                const int t = k / NBINS, b = k - t * NBINS;
-                src = t * NBINS + rot_src(b, rot);
-            }
-            kmap[k] = (short)src;
-        }
-        __syncthreads();
-    }
-    auto issue = [&](int k0, int buf) {
-        const int ch = tid & 7;
-        if (MODE == 1) {
-#pragma unroll 1
-            for (int e = 0; e < 16; ++e) {                    // rolled chroma groups: element-wise gather
-                const int id = tid + 64 * e, row = id >> 4, kk = id & 15;
-                ef_cp_async8(&As[buf][row][kk], Abase + min(m0 + row, M - 1) * dp + (int)kmap[k0 + kk]);
-            }
-        }
-#pragma unroll 1
-        for (int c = 0; c < 8; ++c) {
-            const int row = (tid >> 3) + 8 * c;
-            if (MODE == 0) ef_cp_async16(&As[buf][row][2 * ch], Abase + min(m0 + row, M - 1) * dp + k0 + 2 * ch);
-            ef_cp_async16(&Bs[buf][row][2 * ch], Bbase + min(n0 + row, N - 1) * dp + k0 + 2 * ch);
-        }
-    };
-    // register tile: rows 32 w + rg + 4 i (i = 0..7), columns cg + 8 j (j = 0..7)
-    const int w = tid >> 5, rg = (tid >> 3) & 3, cg = tid & 7;
-    double acc[8][8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i)
-#pragma unroll
-        for (int j = 0; j < 8; ++j) acc[i][j] = 0.0;
-    // ragged edge tiles: a warp whose 32 rows lie past M only helps loading; 8-column groups past N are skipped
-    const bool warp_live = m0 + 32 * w < M;
-    const int jmax = min(8, (N - n0 + 7) >> 3);
-    const int nt = dp / EF_BK;
-    issue(0, 0);
-    asm volatile("cp.async.commit_group;\n" ::: "memory");
-    for (int t = 0; t < nt; ++t) {
-        if (t + 1 < nt) issue((t + 1) * EF_BK, (t + 1) & 1);
-        asm volatile("cp.async.commit_group;\n" ::: "memory");
-        asm volatile("cp.async.wait_group 1;\n" ::: "memory");
-        __syncthreads();
-        const double *Ap = &As[t & 1][32 * w + rg][0];
-        const double *Bp = &Bs[t & 1][cg][0];
-        if (warp_live) {
-            if (jmax == 8) ef_tile_fma<true>(Ap, Bp, 8, acc);    // interior tile: fully unrolled, fragments prefetched
-            else ef_tile_fma<false>(Ap, Bp, jmax, acc);          // ragged right edge: 8-column groups past N skipped
-        }
-        __syncthreads();
-    }
-    double *out = csm + (int64_t)slot * slot_elems;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-        const int row = m0 + 32 * w + rg + 4 * i;
-        if (row >= M) continue;
-        const double sx = (MODE == 0) ? sq[oq + row] : 0.0;
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            const int col = n0 + cg + 8 * j;
-            if (col >= N) continue;
-            double v;
-            if (MODE == 0) {
-                double c2 = __dsub_rn(__dadd_rn(sx, sq[orr + col]), __dmul_rn(2.0, acc[i][j]));
-                c2 = c2 < 0.0 ? 0.0 : c2;
-                v = sqrt(c2);
-            } else {
-                v = __dsub_rn(1.0, acc[i][j]);
-            }
-            out[(int64_t)row * N + col] = v;
-        }
-    }
-}
-
-#endif  // ACOSS_EF_GENERATIONS
-// ---------------------------------------------------------------------------------------------
-// CSM, third generation: the float64 tensor path (DMMA, mma.sync.m8n8k4.f64 — tcgen05 has no float64
-// kind; on sm_100a the legacy warp-level MMA is the only float64 tensor instruction).  ncu on the second
-// generation (profiles/r1_ef_csm.md): FP64 pipe 56 %, two warps per scheduler at 255 registers, stalls are
-// the half-rate DFMA issue itself.  One DMMA replaces 8 DFMA per lane and needs one A and one B double
-// per lane: 64 x 64 CTA tile, 2 x 2 warps of 32 x 32 (4 x 4 MMA tiles, 32 accumulator doubles per lane),
-// 8 LDS.64 per 16 DMMA.  Shared tiles stay row-major [row][k] with a pitch of 20 doubles, so the 4 rows x
-// 4 k a half-warp reads fall in 32 distinct banks.  cp.async two-stage ring as above.
-// ---------------------------------------------------------------------------------------------
-#define EF3_LD 20
 __device__ __forceinline__ void ef_dmma(double &c0, double &c1, double a, double b) {
     asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
                  : "+d"(c0), "+d"(c1)
@@ -433,7 +179,9 @@ __device__ __forceinline__ void ef_quad_dispatch(int imax, int jmax, const doubl
     }
 }
 
-template <int MODE>
+// MODE 0: sqrt(max(0, (|x|^2 + |y|^2) - 2 x.y)); MODE 1: 1 - xhat.yhat with the 12-bin groups of x rolled by oti.
+// WIDE (MODE 1, dp > EF2_MAXDP): the gather computes each rolled source column instead of reading the column map.
+template <int MODE, bool WIDE>
 __global__ void __launch_bounds__(128) ef_csm3_kernel(const double *__restrict__ feat, int dp, int d,
                                                       const double *__restrict__ sq,
                                                       const int64_t *__restrict__ offsets,
@@ -442,7 +190,7 @@ __global__ void __launch_bounds__(128) ef_csm3_kernel(const double *__restrict__
                                                       double *__restrict__ csm, int64_t slot_elems, int tiles_n) {
     __shared__ __align__(16) double As[2][EF_BM][EF3_LD];
     __shared__ __align__(16) double Bs[2][EF_BN][EF3_LD];
-    __shared__ short kmap[MODE == 1 ? EF2_MAXDP : 1];
+    __shared__ short kmap[MODE == 1 && !WIDE ? EF2_MAXDP : 1];
     const int slot = blockIdx.y;
     const int q = pairs[2 * slot], r = pairs[2 * slot + 1];
     const int64_t oq = offsets[q], orr = offsets[r];
@@ -451,16 +199,18 @@ __global__ void __launch_bounds__(128) ef_csm3_kernel(const double *__restrict__
     if (m0 >= M || n0 >= N) return;
     const int tid = threadIdx.x;
     const double *Abase = feat + oq * (int64_t)dp, *Bbase = feat + orr * (int64_t)dp;
-    if (MODE == 1) {                                          // np.roll(X1, oti, axis=2): out[b] = in[(b - oti) mod 12]
-        const int rot = oti_a[slot];
-        for (int k = tid; k < dp; k += 128) {
-            int src = k;
-            if (k < d) {
-                const int t = k / NBINS, b = k - t * NBINS;
-                src = t * NBINS + rot_src(b, rot);
-            }
-            kmap[k] = (short)src;
+    const int rot = MODE == 1 ? oti_a[slot] : 0;
+    // np.roll(X1, oti, axis=2): out[b] = in[(b - oti) mod 12]
+    auto rolled = [&](int k) {
+        int src = k;
+        if (k < d) {
+            const int t = k / NBINS, b = k - t * NBINS;
+            src = t * NBINS + rot_src(b, rot);
         }
+        return src;
+    };
+    if (MODE == 1 && !WIDE) {
+        for (int k = tid; k < dp; k += 128) kmap[k] = (short)rolled(k);
         __syncthreads();
     }
     auto issue = [&](int k0, int buf) {
@@ -469,7 +219,8 @@ __global__ void __launch_bounds__(128) ef_csm3_kernel(const double *__restrict__
 #pragma unroll 1
             for (int e = 0; e < 8; ++e) {                     // rolled chroma groups: element-wise gather
                 const int id = tid + 128 * e, row = id >> 4, kk = id & 15;
-                ef_cp_async8(&As[buf][row][kk], Abase + min(m0 + row, M - 1) * dp + (int)kmap[k0 + kk]);
+                const int src = WIDE ? rolled(k0 + kk) : (int)kmap[k0 + kk];
+                ef_cp_async8(&As[buf][row][kk], Abase + min(m0 + row, M - 1) * dp + src);
             }
         }
 #pragma unroll 1
@@ -530,49 +281,24 @@ __global__ void __launch_bounds__(128) ef_csm3_kernel(const double *__restrict__
     }
 }
 
-static int ef_csm_generation() {
-#ifdef ACOSS_EF_GENERATIONS
-    static int gen = -1;
-    if (gen < 0) {
-        const char *e = getenv("ACOSS_EF_CSM");               // 1 / 2 select the DFMA kernels (A/B timing)
-        gen = (e && e[0] >= '1' && e[0] <= '3') ? e[0] - '0' : 3;
-    }
-    return gen;
-#else
-    return 3;                                                 // the DMMA kernel; ef_csm_kernel only for chroma blocks wider than EF2_MAXDP
-#endif
-}
-
 int launch_ef_csm(int mode, const double *feat, int dp, int d, const double *sq, const int64_t *offsets,
                   const int32_t *pairs, const int32_t *oti, int n, int max_rows, int max_cols, double *csm,
                   int64_t slot_elems, cudaStream_t st) {
     if (n <= 0) return ACOSS_OK;
     const int tiles_m = (max_rows + EF_BM - 1) / EF_BM, tiles_n = (max_cols + EF_BN - 1) / EF_BN;
     dim3 grid((unsigned)(tiles_m * tiles_n), (unsigned)n);
-    if (ef_csm_generation() == 3 && (mode == 0 || dp <= EF2_MAXDP)) {
-        static bool carve[16] = {false};                      // 40 KB static tiles per CTA: ask for the full carve-out
-        int dev = 0;                                          // so that 5 CTAs fit an SM
-        cudaGetDevice(&dev);
-        if (dev >= 0 && dev < 16 && !carve[dev]) {
-            cudaFuncSetAttribute(ef_csm3_kernel<0>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-            cudaFuncSetAttribute(ef_csm3_kernel<1>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-            carve[dev] = true;
-        }
-        if (mode == 0) ef_csm3_kernel<0><<<grid, 128, 0, st>>>(feat, dp, d, sq, offsets, pairs, oti, csm, slot_elems, tiles_n);
-        else ef_csm3_kernel<1><<<grid, 128, 0, st>>>(feat, dp, d, sq, offsets, pairs, oti, csm, slot_elems, tiles_n);
-        CUDA_TRY(cudaGetLastError());
-        return ACOSS_OK;
+    static bool carve[16] = {false};                          // 40 KB static tiles per CTA: ask for the full carve-out
+    int dev = 0;                                              // so that 5 CTAs fit an SM
+    cudaGetDevice(&dev);
+    if (dev >= 0 && dev < 16 && !carve[dev]) {
+        cudaFuncSetAttribute(ef_csm3_kernel<0, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+        cudaFuncSetAttribute(ef_csm3_kernel<1, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+        cudaFuncSetAttribute(ef_csm3_kernel<1, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+        carve[dev] = true;
     }
-#ifdef ACOSS_EF_GENERATIONS
-    if (ef_csm_generation() >= 2 && (mode == 0 || dp <= EF2_MAXDP)) {
-        if (mode == 0) ef_csm2_kernel<0><<<grid, 64, 0, st>>>(feat, dp, d, sq, offsets, pairs, oti, csm, slot_elems, tiles_n);
-        else ef_csm2_kernel<1><<<grid, 64, 0, st>>>(feat, dp, d, sq, offsets, pairs, oti, csm, slot_elems, tiles_n);
-        CUDA_TRY(cudaGetLastError());
-        return ACOSS_OK;
-    }
-#endif
-    if (mode == 0) ef_csm_kernel<0><<<grid, 128, 0, st>>>(feat, dp, d, sq, offsets, pairs, oti, csm, slot_elems, tiles_n);
-    else ef_csm_kernel<1><<<grid, 128, 0, st>>>(feat, dp, d, sq, offsets, pairs, oti, csm, slot_elems, tiles_n);
+    if (mode == 0) ef_csm3_kernel<0, false><<<grid, 128, 0, st>>>(feat, dp, d, sq, offsets, pairs, oti, csm, slot_elems, tiles_n);
+    else if (dp <= EF2_MAXDP) ef_csm3_kernel<1, false><<<grid, 128, 0, st>>>(feat, dp, d, sq, offsets, pairs, oti, csm, slot_elems, tiles_n);
+    else ef_csm3_kernel<1, true><<<grid, 128, 0, st>>>(feat, dp, d, sq, offsets, pairs, oti, csm, slot_elems, tiles_n);
     CUDA_TRY(cudaGetLastError());
     return ACOSS_OK;
 }

@@ -68,14 +68,19 @@ def test_scores_match_reference_golden(eng, gfull, case):
     assert np.array_equal(d["scores"], got[:, 0])
 
 
-@pytest.mark.parametrize("dtype", ["float32", "float64"])
-def test_matrices_match_oracle(eng, dtype):
+ORACLE_DIMS = dict(mfccs=200, ssms=231, chromas=96)
+# chroma blocks padded to 2 064 doubles: wider than the rolled-column map of the chroma contraction (2 048)
+WIDE_CHROMA_DIMS = dict(mfccs=200, ssms=231, chromas=2052)
+
+
+@pytest.mark.parametrize("dtype,dims", [("float32", ORACLE_DIMS), ("float64", ORACLE_DIMS), ("float32", WIDE_CHROMA_DIMS)],
+                         ids=["float32", "float64", "float32-wide_chroma"])
+def test_matrices_match_oracle(eng, dtype, dims):
     """Every stage of one pair against the oracle: OTI, three CSMs, fused matrix, binarisations, scores;
     ragged shapes (rows != columns, neither a multiple of the 64-wide tile)."""
     from acoss_b200 import synthetic
     from oracle import earlyfusion_np as ef
-    feats = synthetic.ef_dataset([2, 1, 1], 150, 411, dims=dict(mfccs=200, ssms=231, chromas=96),
-                                 dtype=np.dtype(dtype), jitter=0.4)
+    feats = synthetic.ef_dataset([2, 1, 1], 150, 411, dims=dims, dtype=np.dtype(dtype), jitter=0.4)
     eng.ef_set_tracks(feats)
     for q, r in [(0, 1), (1, 0), (0, 2), (3, 1)]:
         d = eng.ef_dump_pair(q, r, 0.1, 10)

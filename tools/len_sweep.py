@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Tensor-core vs FFMA2 sweeps by track length (ACOSS_K2_SWEEPS forced, host-to-host score_pairs on slices of the C3 tracks):
-the crossover behind K2_TC_MIN_WINDOWS.  Scores of the two runs must be identical."""
+the crossover behind TC_MIN_WINDOWS.  Scores of the two runs must be identical."""
 import os, sys, time, json
 import numpy as np
 sys.path.insert(0, os.getcwd())
