@@ -66,7 +66,7 @@ struct FastLayout {
     size_t slot_bytes;
     size_t off_hdr, off_rrot, off_aaf, off_bbf, off_aai, off_bbi, off_lo, off_w, off_cb, off_sh, off_cnt,
         off_cand, off_candz, off_zin, off_zout, off_rowpack, off_pool, off_pcnt, off_samp_r, off_samp_c,
-        off_lsel, off_wlist, off_wcnt, off_win, off_qpl, off_rpl;
+        off_lsel, off_wlist, off_wcnt, off_win, off_qpl, off_rpl, off_tcq;
     int max_rows, max_cols, max_frames, lines, pool_cap;
     int plane_frames;                   // frames per byte plane of the tensor sweeps (zero padded past the track end)
     int slog;                           // log2 of the diagonal sampling stride S
@@ -130,6 +130,7 @@ FastLayout make_layout(const SlotGeom &g, int max_frames) {
     L.plane_frames = max_frames + TC_PAD + 16;
     L.off_qpl = take((size_t)3 * L.plane_frames * 16);          // query byte planes [h, l1, l2][frame][16]
     L.off_rpl = take((size_t)3 * L.plane_frames * 16);          // rotated reference byte planes
+    L.off_tcq = take(4 * 4);                                    // next work item of each tensor sweep (slot 0's copy serves the call)
     L.slot_bytes = align_up(o, 256);
     return L;
 }
@@ -238,6 +239,7 @@ __global__ void __launch_bounds__(256) fast_prep_kernel(TrackSet ts, const int32
     uint32_t *cnt = slot_ptr<uint32_t>(scratch, L, slot, L.off_cnt);
     for (int i = threadIdx.x; i < L.lines; i += blockDim.x) cnt[i] = 0u;
     if (threadIdx.x == 0) { *slot_ptr<uint32_t>(scratch, L, slot, L.off_pcnt) = 0u; *slot_ptr<uint32_t>(scratch, L, slot, L.off_wcnt) = 0u; }
+    if (threadIdx.x < 4) slot_ptr<uint32_t>(scratch, L, slot, L.off_tcq)[threadIdx.x] = 0u;
     __syncthreads();
     float *aaf = slot_ptr<float>(scratch, L, slot, L.off_aaf), *bbf = slot_ptr<float>(scratch, L, slot, L.off_bbf);
     int32_t *aai = slot_ptr<int32_t>(scratch, L, slot, L.off_aai), *bbi = slot_ptr<int32_t>(scratch, L, slot, L.off_bbi);
@@ -1516,9 +1518,9 @@ int launch_k2_fast(const TrackSet &ts, const int32_t *pairs, const int32_t *oti,
     auto tb = [&](int id) { if (timer) timer->begin(id); };
     auto te = [&](int id) { if (timer) timer->end(id); };
     tb(K2K_PREP);
-    // Sweeps: tensor cores from TC_MIN_WINDOWS windows on the longer side (a CTA's fixed costs - TMEM allocation, operand
-    // fill, histogram scan - weigh on short lines; measured against the FFMA2 sweeps: +17 % pairs/s at 2 000 frames, level at
-    // 500), FFMA2 below and whenever the features cannot be quantised within the error budget.  ACOSS_K2_SWEEPS=tc|ffma forces one of them (A/B runs, parity tests of both).
+    // Sweeps: tensor cores from TC_MIN_WINDOWS windows on the longer side (a work item's fixed costs - operand fill, histogram
+    // scan - weigh on short lines; measured against the FFMA2 sweeps before the tensor sweeps became persistent: +17 % pairs/s
+    // at 2 000 frames, level at 500), FFMA2 below and whenever the features cannot be quantised within the error budget.  ACOSS_K2_SWEEPS=tc|ffma forces one of them (A/B runs, parity tests of both).
     const char *sweeps_env = getenv("ACOSS_K2_SWEEPS");          // read per call: tests flip it inside one process
     bool use_tc = ts.q_exp >= 0 && std::max(g.max_rows, g.max_cols) >= TC_MIN_WINDOWS;
     if (sweeps_env && sweeps_env[0] == 't') use_tc = ts.q_exp >= 0;
@@ -1577,13 +1579,18 @@ int launch_k2_fast(const TrackSet &ts, const int32_t *pairs, const int32_t *oti,
             CUDA_TRY(cudaFuncSetAttribute(tc_emit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_e));
             tc_attr_done[dev & 63] = true;
         }
-        const unsigned tgc = (unsigned)((int64_t)n * tstrips_c), tgr = (unsigned)((int64_t)n * tstrips_r);
-        // one launch per orientation: a CTA that still holds DENSE2_MIN_LIVE live lines after its sweep sweeps again at once
+        // persistent CTAs, one per SM, taking work items from a counter that fast_prep_kernel zeroed (k2_tc.inl)
+        static int tc_sms[64] = {0};
+        if (!tc_sms[dev & 63]) CUDA_TRY(cudaDeviceGetAttribute(&tc_sms[dev & 63], cudaDevAttrMultiProcessorCount, dev));
+        auto tc_grid = [&](int64_t items) { return (unsigned)std::min<int64_t>(items, tc_sms[dev & 63]); };
+        // one launch per orientation: an item that still holds DENSE2_MIN_LIVE live lines after its sweep is swept again at once
         tb(K2K_HIST_COL);
-        tc_hist_kernel<0><<<tgc, TC_THREADS, smem_h, st>>>(ts, pairs, first, n, L, base, tstrips_c, sh3, status, dbg, dbg + 12, glive, gcap);
+        tc_hist_kernel<0><<<tc_grid((int64_t)n * tstrips_c), TC_THREADS, smem_h, st>>>(ts, pairs, first, n, L, base, tstrips_c, sh3, status, dbg,
+                                                                                       dbg + 12, glive, gcap);
         te(K2K_HIST_COL);
         tb(K2K_HIST_ROW);
-        tc_hist_kernel<1><<<tgr, TC_THREADS, smem_h, st>>>(ts, pairs, first, n, L, base, tstrips_r, sh3, status, dbg + 4, dbg + 16, glive, gcap);
+        tc_hist_kernel<1><<<tc_grid((int64_t)n * tstrips_r), TC_THREADS, smem_h, st>>>(ts, pairs, first, n, L, base, tstrips_r, sh3, status,
+                                                                                       dbg + 4, dbg + 16, glive, gcap);
         CUDA_TRY(cudaGetLastError());
         te(K2K_HIST_ROW);
         const int64_t warps = ((int64_t)gcap + 31) / 32;
@@ -1593,7 +1600,8 @@ int launch_k2_fast(const TrackSet &ts, const int32_t *pairs, const int32_t *oti,
         te(K2K_SPARSE);
         const int groups = std::max(tstrips_c, (g.words + 3) / 4);
         tb(K2K_EMIT);
-        tc_emit_kernel<<<(unsigned)((int64_t)n * groups), TC_THREADS, smem_e, st>>>(ts, pairs, first, n, L, base, groups, sh3, crp, g.words, g.crp_words);
+        tc_emit_kernel<<<tc_grid((int64_t)n * groups), TC_THREADS, smem_e, st>>>(ts, pairs, first, n, L, base, groups, sh3, crp, g.words,
+                                                                                 g.crp_words);
         CUDA_TRY(cudaGetLastError());
         te(K2K_EMIT);
     } else {
