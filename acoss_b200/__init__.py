@@ -3,5 +3,6 @@ hot path (OTI -> HPCP cross-similarity -> binary CRP -> Qmax / Smith-Waterman), 
 reference's CoverAlgorithm plugin API.  See DESIGN.md."""
 from ._lib import AcossError, Params, default_params  # noqa: F401
 from .engine import Engine, pack_tracks  # noqa: F401
+from .simple import Simple  # noqa: F401
 
 __version__ = "0.1.0"

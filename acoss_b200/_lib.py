@@ -33,6 +33,12 @@ class Params(C.Structure):
                 ("f5_asymmetric", C.c_int32)]
 
 
+class SimpleParams(C.Structure):
+    """Mirror of ``acoss_simple_params`` (include/acoss_b200.h)."""
+    _fields_ = [("m", C.c_int32), ("oti", C.c_int32), ("s2_squared", C.c_int32), ("s3_positive", C.c_int32),
+                ("s4_roll_first", C.c_int32)]
+
+
 _lib = None
 
 # name -> (restype, argtypes); every symbol include/acoss_b200.h declares
@@ -67,6 +73,11 @@ SIGNATURES = {
     "acoss_ef_dump_pair": (C.c_int, [_vp, C.c_int32, C.c_int32, C.c_double, C.c_int32, _i32p, _vp, _vp, _fp]),
     "acoss_ef_stage_ms": (C.c_int, [_vp, _vp]),
     "acoss_ef_last_stats": (C.c_int, [_vp, _i64p]),
+    "acoss_set_tracks_pooled": (C.c_int, [_vp, _fp, _i64p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _i64p]),
+    "acoss_simple_default_params": (None, [C.POINTER(SimpleParams)]),
+    "acoss_simple_score_pairs": (C.c_int, [_vp, _i32p, C.c_int64, C.POINTER(SimpleParams), _fp]),
+    "acoss_simple_score_pairs_device": (C.c_int, [_vp, _i32p, C.c_int64, C.POINTER(SimpleParams), _fp]),
+    "acoss_simple_dump_pair": (C.c_int, [_vp, C.c_int32, C.c_int32, C.POINTER(SimpleParams), _i32p, _vp, _i32p, _fp]),
 }
 
 
@@ -99,4 +110,15 @@ def default_params(**overrides) -> Params:
         if not hasattr(p, k):
             raise TypeError("unknown parameter %r" % k)
         setattr(p, k, v)
+    return p
+
+
+def simple_default_params(**overrides) -> SimpleParams:
+    """acoss_simple_default_params (m = 10, oti = 1, S2 = S3 = S4 = 0) with keyword overrides."""
+    p = SimpleParams()
+    load().acoss_simple_default_params(C.byref(p))
+    for k, v in overrides.items():
+        if not hasattr(p, k):
+            raise TypeError("unknown parameter %r" % k)
+        setattr(p, k, int(v))
     return p

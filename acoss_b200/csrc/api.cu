@@ -10,6 +10,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <functional>
 #include <vector>
 
 #include "common.cuh"
@@ -76,6 +77,8 @@ struct acoss_ctx {
     int32_t ef_d[3] = {0, 0, 0}, ef_dp[3] = {0, 0, 0};
     int32_t ef_tracks = 0;
     Buf ef_csm, ef_stat, ef_shapes, ef_nn, ef_csmoff, ef_oti, ef_pairs, ef_scores, ef_bits, ef_bitoff, ef_stage;
+    // SiMPle pair scoring (acoss_simple_*): per-slot workspace, pair list / scores / OTI of the host entry points
+    Buf sp_ws, sp_pairs, sp_scores, sp_oti;
     int64_t ef_stats[4] = {0, 0, 0, 0};
 };
 
@@ -201,7 +204,8 @@ int acoss_destroy(acoss_ctx *c) {
                    &c->rrot, &c->aa, &c->bb, &c->D, &c->halo, &c->misc, &c->fast, &c->fbmap, &c->dbg, &c->glive, &c->fbtmp,
                    &c->ef_feat[0], &c->ef_feat[1], &c->ef_feat[2], &c->ef_sq[0], &c->ef_sq[1], &c->ef_cmed, &c->ef_off,
                    &c->ef_csm, &c->ef_stat, &c->ef_shapes, &c->ef_nn, &c->ef_csmoff, &c->ef_oti, &c->ef_pairs,
-                   &c->ef_scores, &c->ef_bits, &c->ef_bitoff, &c->ef_stage};
+                   &c->ef_scores, &c->ef_bits, &c->ef_bitoff, &c->ef_stage, &c->sp_ws, &c->sp_pairs, &c->sp_scores,
+                   &c->sp_oti};
     for (Buf *b : bufs) free_buf(*b);
     if (c->own_frames && c->d_frames) cudaFree(c->d_frames);
     if (c->d_offsets) cudaFree(c->d_offsets);
@@ -292,6 +296,40 @@ static int finish_tracks(acoss_ctx *c, const int64_t *offsets, int32_t n_tracks,
     return ACOSS_OK;
 }
 
+// common tail of acoss_set_tracks_raw / acoss_set_tracks_pooled: uploads the raw frames, runs `reduce` (raw, raw
+// offsets, output offsets, output frames: device) into the new resident set and finishes it; off = output offsets
+using RawReduce = std::function<int(const float *, const int64_t *, const int64_t *, int64_t, float *)>;
+static int reduce_raw_tracks(acoss_ctx *c, const float *raw_frames, const int64_t *raw_offsets, int32_t n_tracks,
+                             const std::vector<int64_t> &off, int64_t mx, int64_t mn, int64_t *offsets_out,
+                             const RawReduce &reduce) {
+    const int64_t total_raw = raw_offsets[n_tracks], total = off[n_tracks];
+    if (c->own_frames && c->d_frames) CUDA_TRY(cudaFree(c->d_frames));
+    c->d_frames = nullptr;
+    if (c->d_offsets) CUDA_TRY(cudaFree(c->d_offsets));
+    if (c->d_gchroma) CUDA_TRY(cudaFree(c->d_gchroma));
+    c->d_offsets = nullptr; c->d_gchroma = nullptr;
+    float *d_raw = nullptr;
+    int64_t *d_roff = nullptr, *d_ooff = nullptr;
+    auto cleanup = [&]() { if (d_raw) cudaFree(d_raw); if (d_roff) cudaFree(d_roff); if (d_ooff) cudaFree(d_ooff); };
+#define CUDA_TRYC(x) do { cudaError_t _e = (x); if (_e != cudaSuccess) { acoss_set_error("%s -> %s", #x, cudaGetErrorString(_e)); cleanup(); return _e == cudaErrorMemoryAllocation ? ACOSS_E_NOMEM : ACOSS_E_CUDA; } } while (0)
+    CUDA_TRYC(cudaMalloc((void **)&d_raw, (size_t)std::max<int64_t>(total_raw, 1) * NBINS * sizeof(float)));
+    CUDA_TRYC(cudaMalloc((void **)&d_roff, (size_t)(n_tracks + 1) * sizeof(int64_t)));
+    CUDA_TRYC(cudaMalloc((void **)&d_ooff, (size_t)(n_tracks + 1) * sizeof(int64_t)));
+    CUDA_TRYC(cudaMalloc((void **)&c->d_frames, (size_t)(total * NBINS + 64) * sizeof(float)));
+    c->own_frames = true;
+    CUDA_TRYC(cudaMemsetAsync(c->d_frames + total * NBINS, 0, 64 * sizeof(float), c->stream));
+    CUDA_TRYC(cudaMemcpyAsync(d_raw, raw_frames, (size_t)total_raw * NBINS * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRYC(cudaMemcpyAsync(d_roff, raw_offsets, (size_t)(n_tracks + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRYC(cudaMemcpyAsync(d_ooff, off.data(), (size_t)(n_tracks + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, c->stream));
+    int rc = reduce(d_raw, d_roff, d_ooff, total, c->d_frames);
+    if (rc == ACOSS_OK) { cudaError_t e = cudaStreamSynchronize(c->stream); if (e != cudaSuccess) { acoss_set_error("on-ramp: %s", cudaGetErrorString(e)); rc = ACOSS_E_CUDA; } }
+    cleanup();
+#undef CUDA_TRYC
+    if (rc != ACOSS_OK) return rc;
+    if (offsets_out) memcpy(offsets_out, off.data(), (size_t)(n_tracks + 1) * sizeof(int64_t));
+    return finish_tracks(c, off.data(), n_tracks, mx, mn);
+}
+
 int acoss_set_tracks_raw(acoss_ctx *c, const float *raw_frames, const int64_t *raw_offsets, int32_t n_tracks,
                          int32_t downsample_fac, int64_t *offsets_out) {
     if (!c || !raw_frames || !raw_offsets || n_tracks <= 0) { acoss_set_error("set_tracks_raw: bad arguments"); return ACOSS_E_INVALID; }
@@ -313,32 +351,40 @@ int acoss_set_tracks_raw(acoss_ctx *c, const float *raw_frames, const int64_t *r
         mn = std::min(mn, no);
     }
     if (mx > (1 << 20)) { acoss_set_error("set_tracks_raw: track longer than 2^20 frames"); return ACOSS_E_INVALID; }
-    const int64_t total_raw = raw_offsets[n_tracks], total = off[n_tracks];
-    if (c->own_frames && c->d_frames) CUDA_TRY(cudaFree(c->d_frames));
-    c->d_frames = nullptr;
-    if (c->d_offsets) CUDA_TRY(cudaFree(c->d_offsets));
-    if (c->d_gchroma) CUDA_TRY(cudaFree(c->d_gchroma));
-    c->d_offsets = nullptr; c->d_gchroma = nullptr;
-    float *d_raw = nullptr;
-    int64_t *d_roff = nullptr, *d_ooff = nullptr;
-    auto cleanup = [&]() { if (d_raw) cudaFree(d_raw); if (d_roff) cudaFree(d_roff); if (d_ooff) cudaFree(d_ooff); };
-#define CUDA_TRYC(x) do { cudaError_t _e = (x); if (_e != cudaSuccess) { acoss_set_error("%s -> %s", #x, cudaGetErrorString(_e)); cleanup(); return _e == cudaErrorMemoryAllocation ? ACOSS_E_NOMEM : ACOSS_E_CUDA; } } while (0)
-    CUDA_TRYC(cudaMalloc((void **)&d_raw, (size_t)std::max<int64_t>(total_raw, 1) * NBINS * sizeof(float)));
-    CUDA_TRYC(cudaMalloc((void **)&d_roff, (size_t)(n_tracks + 1) * sizeof(int64_t)));
-    CUDA_TRYC(cudaMalloc((void **)&d_ooff, (size_t)(n_tracks + 1) * sizeof(int64_t)));
-    CUDA_TRYC(cudaMalloc((void **)&c->d_frames, (size_t)(total * NBINS + 64) * sizeof(float)));
-    c->own_frames = true;
-    CUDA_TRYC(cudaMemsetAsync(c->d_frames + total * NBINS, 0, 64 * sizeof(float), c->stream));
-    CUDA_TRYC(cudaMemcpyAsync(d_raw, raw_frames, (size_t)total_raw * NBINS * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-    CUDA_TRYC(cudaMemcpyAsync(d_roff, raw_offsets, (size_t)(n_tracks + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, c->stream));
-    CUDA_TRYC(cudaMemcpyAsync(d_ooff, off.data(), (size_t)(n_tracks + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, c->stream));
-    int rc = launch_median_sync(d_raw, d_roff, d_ooff, n_tracks, downsample_fac, total, c->d_frames, c->stream);
-    if (rc == ACOSS_OK) { cudaError_t e = cudaStreamSynchronize(c->stream); if (e != cudaSuccess) { acoss_set_error("median_sync: %s", cudaGetErrorString(e)); rc = ACOSS_E_CUDA; } }
-    cleanup();
-#undef CUDA_TRYC
-    if (rc != ACOSS_OK) return rc;
-    if (offsets_out) memcpy(offsets_out, off.data(), (size_t)(n_tracks + 1) * sizeof(int64_t));
-    return finish_tracks(c, off.data(), n_tracks, mx, mn);
+    return reduce_raw_tracks(c, raw_frames, raw_offsets, n_tracks, off, mx, mn, offsets_out,
+                             [&](const float *raw, const int64_t *roff, const int64_t *ooff, int64_t total, float *out) {
+                                 return launch_median_sync(raw, roff, ooff, n_tracks, downsample_fac, total, out, c->stream);
+                             });
+}
+
+int acoss_set_tracks_pooled(acoss_ctx *c, const float *raw_frames, const int64_t *raw_offsets, int32_t n_tracks,
+                            int32_t win, int32_t skip, int32_t keep_partial, int64_t *offsets_out) {
+    if (!c || !raw_frames || !raw_offsets || n_tracks <= 0) { acoss_set_error("set_tracks_pooled: bad arguments"); return ACOSS_E_INVALID; }
+    if (win < 1 || win > 65536 || skip < 1 || skip > 65536) { acoss_set_error("set_tracks_pooled: win and skip must be in 1..65536"); return ACOSS_E_INVALID; }
+    CUDA_TRY(cudaSetDevice(c->device));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
+    if (raw_offsets[0] != 0) { acoss_set_error("set_tracks_pooled: offsets must start at 0"); return ACOSS_E_INVALID; }
+    std::vector<int64_t> off(n_tracks + 1, 0);
+    int64_t mx = 0, mn = INT64_MAX;
+    for (int t = 0; t < n_tracks; ++t) {
+        const int64_t n = raw_offsets[t + 1] - raw_offsets[t];
+        if (n < 0) { acoss_set_error("set_tracks_pooled: offsets must be non-decreasing"); return ACOSS_E_INVALID; }
+        int64_t no;
+        if (!keep_partial) {                                     // S5 default: full windows only
+            if (n < win) { acoss_set_error("set_tracks_pooled: track %d has %lld raw frames, fewer than win = %d", t, (long long)n, win); return ACOSS_E_TOO_SHORT; }
+            no = (n - win) / skip + 1;
+        } else {                                                 // S5 = 1: a shorter last window covers the tail
+            no = n <= win ? (n > 0 ? 1 : 0) : (n - win + skip - 1) / skip + 1;
+        }
+        off[t + 1] = off[t] + no;
+        mx = std::max(mx, no);
+        mn = std::min(mn, no);
+    }
+    if (mx > (1 << 20)) { acoss_set_error("set_tracks_pooled: track longer than 2^20 pooled frames"); return ACOSS_E_INVALID; }
+    return reduce_raw_tracks(c, raw_frames, raw_offsets, n_tracks, off, mx, mn, offsets_out,
+                             [&](const float *raw, const int64_t *roff, const int64_t *ooff, int64_t total, float *out) {
+                                 return launch_mean_pool(raw, roff, ooff, n_tracks, win, skip, total, out, c->stream);
+                             });
 }
 
 int acoss_get_tracks(acoss_ctx *c, float *frames_out, int64_t total_frames) {
@@ -1081,6 +1127,111 @@ int acoss_ef_stage_ms(acoss_ctx *c, double ms[5]) {
 int acoss_ef_last_stats(acoss_ctx *c, int64_t stats[4]) {
     if (!c || !stats) { acoss_set_error("ef_last_stats: NULL argument"); return ACOSS_E_INVALID; }
     memcpy(stats, c->ef_stats, sizeof(c->ef_stats));
+    return ACOSS_OK;
+}
+
+// ---- Simple (SiMPle) pair scoring -------------------------------------------------------------------------------
+
+void acoss_simple_default_params(acoss_simple_params *p) {
+    if (!p) return;
+    p->m = 10; p->oti = 1; p->s2_squared = 0; p->s3_positive = 0; p->s4_roll_first = 0;
+}
+
+static int simple_check(const acoss_ctx *c, const acoss_simple_params *p) {
+    if (!c || !p) { acoss_set_error("NULL context or params"); return ACOSS_E_INVALID; }
+    if (!c->d_frames) { acoss_set_error("no tracks resident: call acoss_set_tracks_pooled first"); return ACOSS_E_INVALID; }
+    if (p->m < 1 || p->m > 128) { acoss_set_error("subsequence length m = %d outside 1..128", p->m); return ACOSS_E_INVALID; }
+    if (c->min_frames < p->m) {
+        acoss_set_error("a track has %d pooled frames, fewer than the subsequence length m = %d", c->min_frames, p->m);
+        return ACOSS_E_TOO_SHORT;
+    }
+    return ACOSS_OK;
+}
+
+// Enqueues the scoring of K pairs (device list) in workspace-limited chunks; oti_dev (may be NULL) receives the OTIs,
+// prof0 / idx0 (may be NULL) the profile and index arrays of workspace slot 0 (the first pair of the last chunk).
+static int simple_run(acoss_ctx *c, const int32_t *pairs_dev, int64_t K, const acoss_simple_params *p, float *scores_dev,
+                      int32_t *oti_dev, const double **prof0 = nullptr, const int32_t **idx0 = nullptr) {
+    TRY(simple_check(c, p));
+    if (K <= 0) return ACOSS_OK;
+    CUDA_TRY(cudaSetDevice(c->device));
+    const size_t per_slot = simple_slot_bytes(c->max_frames, p->m);
+    const int64_t slots = std::max<int64_t>(1, std::min<int64_t>({K, (int64_t)8192, c->ws_limit / (int64_t)per_slot}));
+    TRY(ensure(c->sp_ws, (size_t)slots * per_slot));
+    const int64_t rows = std::max(1, c->max_frames - p->m + 1);
+    SimpleArgs a;
+    a.frames = c->d_frames; a.offsets = c->d_offsets; a.pairs = pairs_dev;
+    a.m = p->m; a.oti = p->oti ? 1 : 0; a.s2_squared = p->s2_squared ? 1 : 0; a.s3_positive = p->s3_positive ? 1 : 0;
+    a.s4_roll_first = p->s4_roll_first ? 1 : 0;
+    a.max_frames = c->max_frames;
+    a.stage_pitch = (int64_t)2 * c->max_frames * NBINS;
+    a.row_pitch = rows;
+    char *w = (char *)c->sp_ws.p;                                 // [stage][thr][cnt][prof][idx][cand], each slots x pitch
+    a.stage = (float *)w; w += (size_t)slots * a.stage_pitch * 4;
+    a.prof = (double *)w; w += (size_t)slots * rows * 8;
+    a.thr = (uint32_t *)w; w += (size_t)slots * rows * 4;
+    a.cnt = (int32_t *)w; w += (size_t)slots * rows * 4;
+    a.idx = (int32_t *)w; w += (size_t)slots * rows * 4;
+    a.cand = (int32_t *)w;
+    a.scores = scores_dev; a.oti_out = oti_dev;
+    if (prof0) *prof0 = a.prof;
+    if (idx0) *idx0 = a.idx;
+    for (int64_t first = 0; first < K; first += slots) {
+        a.first = first;
+        TRY(launch_simple_pairs(a, (int)std::min<int64_t>(slots, K - first), c->stream));
+    }
+    return ACOSS_OK;
+}
+
+static int simple_pairs_in_range(const acoss_ctx *c, const int32_t *pairs, int64_t K) {
+    for (int64_t k = 0; k < 2 * K; ++k)
+        if (pairs[k] < 0 || pairs[k] >= c->n_tracks) { acoss_set_error("pair index %d out of range", pairs[k]); return ACOSS_E_INVALID; }
+    return ACOSS_OK;
+}
+
+int acoss_simple_score_pairs(acoss_ctx *c, const int32_t *pairs, int64_t K, const acoss_simple_params *p, float *scores) {
+    if (!c || (K > 0 && (!pairs || !scores))) { acoss_set_error("simple_score_pairs: NULL argument"); return ACOSS_E_INVALID; }
+    TRY(simple_check(c, p));
+    if (K <= 0) return ACOSS_OK;
+    TRY(simple_pairs_in_range(c, pairs, K));
+    CUDA_TRY(cudaSetDevice(c->device));
+    TRY(ensure(c->sp_pairs, (size_t)K * 8));
+    TRY(ensure(c->sp_scores, (size_t)K * 4));
+    CUDA_TRY(cudaMemcpyAsync(c->sp_pairs.p, pairs, (size_t)K * 8, cudaMemcpyHostToDevice, c->stream));
+    TRY(simple_run(c, (const int32_t *)c->sp_pairs.p, K, p, (float *)c->sp_scores.p, nullptr));
+    CUDA_TRY(cudaMemcpyAsync(scores, c->sp_scores.p, (size_t)K * 4, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
+    return ACOSS_OK;
+}
+
+int acoss_simple_score_pairs_device(acoss_ctx *c, const int32_t *pairs_dev, int64_t K, const acoss_simple_params *p,
+                                    float *scores_dev) {
+    if (!c || (K > 0 && (!pairs_dev || !scores_dev))) { acoss_set_error("simple_score_pairs_device: NULL argument"); return ACOSS_E_INVALID; }
+    return simple_run(c, pairs_dev, K, p, scores_dev, nullptr);
+}
+
+int acoss_simple_dump_pair(acoss_ctx *c, int32_t q, int32_t r, const acoss_simple_params *p, int32_t *oti,
+                           double *profile, int32_t *index, float *score) {
+    TRY(simple_check(c, p));
+    const int32_t pr[2] = {q, r};
+    TRY(simple_pairs_in_range(c, pr, 1));
+    CUDA_TRY(cudaSetDevice(c->device));
+    TRY(ensure(c->sp_pairs, 8));
+    TRY(ensure(c->sp_scores, 4));
+    TRY(ensure(c->sp_oti, 4));
+    CUDA_TRY(cudaMemcpyAsync(c->sp_pairs.p, pr, 8, cudaMemcpyHostToDevice, c->stream));
+    const double *prof = nullptr;
+    const int32_t *idx = nullptr;
+    TRY(simple_run(c, (const int32_t *)c->sp_pairs.p, 1, p, (float *)c->sp_scores.p, (int32_t *)c->sp_oti.p, &prof, &idx));
+    int64_t hoff[2];
+    CUDA_TRY(cudaMemcpyAsync(hoff, c->d_offsets + q, 16, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
+    const int64_t rows = hoff[1] - hoff[0] - p->m + 1;          // profile length of the query
+    if (profile) CUDA_TRY(cudaMemcpyAsync(profile, prof, (size_t)rows * 8, cudaMemcpyDeviceToHost, c->stream));
+    if (index) CUDA_TRY(cudaMemcpyAsync(index, idx, (size_t)rows * 4, cudaMemcpyDeviceToHost, c->stream));
+    if (oti) CUDA_TRY(cudaMemcpyAsync(oti, c->sp_oti.p, 4, cudaMemcpyDeviceToHost, c->stream));
+    if (score) CUDA_TRY(cudaMemcpyAsync(score, c->sp_scores.p, 4, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
     return ACOSS_OK;
 }
 

@@ -139,6 +139,34 @@ int launch_knn_rows(const double *csms, const int64_t *offsets, const int32_t *s
                     int max_rows, int max_cols, uint32_t *bits_dp, int64_t slot_words, int wpr, uint32_t *bits_out,
                     const int64_t *out_offsets, int32_t *rows, int32_t *cols, cudaStream_t st);
 
+// K0: mean pooling of raw frames (the SiMPle on-ramp): out frame k of a track = mean of raw frames
+// [k*skip, min(k*skip + win, n)), sequential float32 sum, one float32 division
+int launch_mean_pool(const float *raw, const int64_t *raw_off, const int64_t *out_off, int n_tracks, int win, int skip,
+                     int64_t total_out, float *out, cudaStream_t st);
+
+// K6: SiMPle pair scoring (k6_simple.cu), one CTA per pair of pairs[first .. first + n) in workspace slots 0 .. n-1
+#define SIMPLE_CAND 32        // listed candidate cells per profile row; a row with more is evaluated over all j
+struct SimpleArgs {
+    const float *frames;      // resident track set
+    const int64_t *offsets;
+    const int32_t *pairs;     // device, absolute pair indices
+    int64_t first;
+    int32_t m, oti, s2_squared, s3_positive, s4_roll_first;
+    int32_t max_frames;
+    float *stage;             // [slot][2][max_frames][12] both tracks of the pair, rolled
+    int64_t stage_pitch;      // floats per slot
+    uint32_t *thr;            // [slot][row_pitch] row minima, then candidate thresholds (fixed point)
+    int32_t *cnt;             // [slot][row_pitch] candidates per row
+    int32_t *cand;            // [slot][row_pitch][SIMPLE_CAND] candidate columns
+    double *prof;             // [slot][row_pitch] matrix profile
+    int32_t *idx;             // [slot][row_pitch] profile index
+    int64_t row_pitch;
+    float *scores;            // [pair]
+    int32_t *oti_out;         // [pair] or NULL
+};
+size_t simple_slot_bytes(int max_frames, int m);
+int launch_simple_pairs(const SimpleArgs &args, int n, cudaStream_t st);
+
 // EarlyFusion stages (k5_earlyfusion.cu)
 int launch_ef_widen(const void *src, int elem_size, int64_t rows, int d, int dp, double *dst, cudaStream_t st);
 int launch_ef_rownorm(double *feat, int64_t rows, int dp, int mode, double *sq, cudaStream_t st);

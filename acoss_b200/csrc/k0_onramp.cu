@@ -1,4 +1,4 @@
-// K0 — feature on-ramp: median downsampling of raw HPCP frames on the GPU.
+// K0 — feature on-ramp: median downsampling (Serra09) and mean pooling (SiMPle) of raw HPCP frames on the GPU.
 //
 // Replaces the aggregation inside Serra09.load_features / ChenFusion.load_features
 //   /root/reference/acoss/algorithms/rqa_serra09.py:47-53
@@ -62,7 +62,42 @@ __global__ void __launch_bounds__(32 * ONRAMP_WPC) median_sync_kernel(const floa
     }
 }
 
+// Mean pooling (the SiMPle on-ramp, simple_silva.py:38-41): output frame k of a track is the per-bin mean of raw
+// frames [k*skip, min(k*skip + win, n)) as np.mean(X[a:b], axis=0) computes it on C-contiguous float32 data: a
+// sequential float32 sum in frame order, then one float32 division by the frame count.  One warp per output frame,
+// lanes 0..11 own the bins (one 48 B frame per step: coalesced).
+__global__ void __launch_bounds__(32 * ONRAMP_WPC) mean_pool_kernel(const float *__restrict__ raw,
+                                                                  const int64_t *__restrict__ raw_off,
+                                                                  const int64_t *__restrict__ out_off,
+                                                                  int n_tracks, int win, int skip,
+                                                                  float *__restrict__ out) {
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t f = (int64_t)blockIdx.x * ONRAMP_WPC + warp;
+    if (f >= out_off[n_tracks] || lane >= NBINS) return;
+    int lo = 0, hi = n_tracks - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (out_off[mid] <= f) lo = mid; else hi = mid - 1;
+    }
+    const int64_t k = f - out_off[lo];
+    const int64_t n_raw = raw_off[lo + 1] - raw_off[lo];
+    const int64_t L = min((int64_t)win, n_raw - k * skip);
+    const float *src = raw + (raw_off[lo] + k * skip) * NBINS + lane;
+    float acc = 0.f;
+    for (int64_t r = 0; r < L; ++r) acc = __fadd_rn(acc, __ldg(src + r * NBINS));
+    out[f * NBINS + lane] = __fdiv_rn(acc, (float)L);
+}
+
 }  // namespace
+
+int launch_mean_pool(const float *raw, const int64_t *raw_off, const int64_t *out_off, int n_tracks, int win, int skip,
+                     int64_t total_out, float *out, cudaStream_t st) {
+    if (total_out <= 0) return ACOSS_OK;
+    const int64_t blocks = (total_out + ONRAMP_WPC - 1) / ONRAMP_WPC;
+    mean_pool_kernel<<<(unsigned)blocks, 32 * ONRAMP_WPC, 0, st>>>(raw, raw_off, out_off, n_tracks, win, skip, out);
+    CUDA_TRY(cudaGetLastError());
+    return ACOSS_OK;
+}
 
 int onramp_max_fac() { return ONRAMP_MAX_FAC; }
 

@@ -11,6 +11,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import ALIGN_DMAX, ALIGN_DMAX_PLAIN, ALIGN_QMAX, ALIGN_SW, AcossError, Params, check, default_params  # noqa: F401
+from ._lib import SimpleParams, simple_default_params  # noqa: F401
 
 __all__ = ["Engine", "AcossError", "default_params", "pack_tracks"]
 
@@ -91,6 +92,23 @@ class Engine:
         out_off = np.zeros(n + 1, dtype=np.int64)
         check(self._lib.acoss_set_tracks_raw(self._ctx, raw_frames.ctypes.data, raw_offsets.ctypes.data, n,
                                              int(downsample_fac), out_off.ctypes.data))
+        self._keepalive = None
+        self.n_tracks = n
+        self.offsets = out_off
+        return out_off
+
+    def set_tracks_pooled(self, raw_frames, raw_offsets, win: int = 200, skip: int = 100,
+                          keep_partial: bool = False) -> np.ndarray:
+        """Raw chroma frames -> GPU mean pooling (acoss_set_tracks_pooled, the pooling of simple_silva.py:38-41) ->
+        resident track set.  keep_partial is switch S5.  Returns the pooled offsets."""
+        raw_offsets = np.ascontiguousarray(raw_offsets, dtype=np.int64)
+        raw_frames = np.ascontiguousarray(raw_frames, dtype=np.float32)
+        n = len(raw_offsets) - 1
+        if raw_frames.size != int(raw_offsets[-1]) * 12:
+            raise ValueError("frames size does not match offsets")
+        out_off = np.zeros(n + 1, dtype=np.int64)
+        check(self._lib.acoss_set_tracks_pooled(self._ctx, raw_frames.ctypes.data, raw_offsets.ctypes.data, n,
+                                                int(win), int(skip), int(bool(keep_partial)), out_off.ctypes.data))
         self._keepalive = None
         self.n_tracks = n
         self.offsets = out_off
@@ -223,6 +241,35 @@ class Engine:
         check(self._lib.acoss_last_stats(self._ctx, st.ctypes.data))
         return dict(pairs=int(st[0]), fallback_pairs=int(st[1]), launches=int(st[2]), cells=int(st[3]),
                     exact_cells=int(st[4]), status_or=int(st[5]), chunks=int(st[6]))
+
+    # -- Simple (SiMPle) pair scoring ----------------------------------------------------------------
+    def simple_score_pairs(self, pairs, params: SimpleParams | None = None) -> np.ndarray:
+        """pairs (K, 2) int -> float32 (K,): the values Simple.similarity stores (acoss_simple_score_pairs)."""
+        params = params or simple_default_params()
+        pairs = np.ascontiguousarray(pairs, dtype=np.int32).reshape(-1, 2)
+        out = np.empty(len(pairs), dtype=np.float32)
+        check(self._lib.acoss_simple_score_pairs(self._ctx, pairs.ctypes.data, len(pairs), C.byref(params),
+                                                 out.ctypes.data))
+        return out
+
+    def simple_score_pairs_device(self, pairs_ptr: int, n_pairs: int, scores_ptr: int,
+                                  params: SimpleParams | None = None):
+        """Device in / device out, asynchronous on the engine stream; call sync()."""
+        params = params or simple_default_params()
+        check(self._lib.acoss_simple_score_pairs_device(self._ctx, pairs_ptr, int(n_pairs), C.byref(params),
+                                                        scores_ptr))
+
+    def simple_dump_pair(self, q: int, r: int, params: SimpleParams | None = None) -> dict:
+        """-> dict(oti, profile float64 (n_q - m + 1,), index int32, score float32) of one pair."""
+        params = params or simple_default_params()
+        rows = max(int(self.offsets[q + 1] - self.offsets[q]) - int(params.m) + 1, 0)
+        oti = C.c_int32(0)
+        score = C.c_float(0)
+        prof = np.zeros(max(rows, 1), dtype=np.float64)
+        idx = np.zeros(max(rows, 1), dtype=np.int32)
+        check(self._lib.acoss_simple_dump_pair(self._ctx, int(q), int(r), C.byref(params), C.addressof(oti),
+                                               prof.ctypes.data, idx.ctypes.data, C.addressof(score)))
+        return dict(oti=int(oti.value), profile=prof[:rows], index=idx[:rows], score=np.float32(score.value))
 
     # -- EarlyFusion pair scoring ---------------------------------------------------------------
     EF_KINDS = ("mfccs", "ssms", "chromas", "early")

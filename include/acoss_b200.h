@@ -179,6 +179,45 @@ int acoss_ef_score_pairs(acoss_ctx *ctx, const int32_t *pairs, int64_t n_pairs, 
 int acoss_ef_dump_pair(acoss_ctx *ctx, int32_t q, int32_t r, double kappa, int32_t K, int32_t *oti, double *csms,
                        uint32_t *bits, float *scores);
 
+/* ---- Simple (SiMPle) pair scoring (simple_silva.py:17-126) ----------------------------------------------------
+ * Parity is unpinned against the reference and pinned against the restatement of DESIGN.md §2 (switches S1-S5),
+ * which oracle/simple_np.py implements. */
+
+/* Replaces the mean pooling of Simple.load_features (simple_silva.py:38-41): pooled frame k of a track is the
+ * per-bin mean of raw frames [k*skip, k*skip + win) (a sequential float32 sum, one float32 division: np.mean on
+ * float32), computed on the GPU; the pooled tracks become the resident set and acoss_get_tracks reads them back.
+ * keep_partial = 0 (S5 default): only full windows, (n - win)/skip + 1 frames, and a track with n < win is
+ * ACOSS_E_TOO_SHORT.  keep_partial = 1: one more, shorter window [k*skip, n) covers a tail the full windows miss (a
+ * track with 1 <= n <= win gives one frame).  raw_frames / raw_offsets: host memory, layout of acoss_set_tracks.
+ * offsets_out (may be NULL, n_tracks + 1 entries) receives the pooled offsets.  win, skip in 1..65536. */
+int acoss_set_tracks_pooled(acoss_ctx *ctx, const float *raw_frames, const int64_t *raw_offsets, int32_t n_tracks,
+                            int32_t win, int32_t skip, int32_t keep_partial, int64_t *offsets_out);
+
+typedef struct acoss_simple_params {
+    int32_t m;              /* S1: subsequence length in pooled frames, 10 (unconfirmed against the reference); 1..128 */
+    int32_t oti;            /* 1: transpose by the optimal transposition index (simple_silva.py:45-54)                  */
+    int32_t s2_squared;     /* S2: 1 = the profile keeps squared distances (default 0: d = sqrt(d2))                   */
+    int32_t s3_positive;    /* S3: 1 = score = +median (default 0: -median, so that higher means more similar)         */
+    int32_t s4_roll_first;  /* S4: 1 = the query is rolled, oti = argmax <roll(g_q, s), g_r> (get_oti); default 0 rolls */
+                            /*     the reference, oti = argmax <g_q, roll(g_r, s)> (essentia)                             */
+} acoss_simple_params;
+
+/* Fills *p with the defaults: m = 10, oti = 1, S2 = S3 = S4 = 0. */
+void acoss_simple_default_params(acoss_simple_params *p);
+
+/* Replaces Simple.similarity(idxs) for a whole batch: scores[k] = the float stored in Ds["main"][q][r] for
+ * pairs[2k] = q (query), pairs[2k+1] = r.  Host buffers.  ACOSS_E_TOO_SHORT when a resident track has fewer than m
+ * frames, ACOSS_E_INVALID for m outside 1..128. */
+int acoss_simple_score_pairs(acoss_ctx *ctx, const int32_t *pairs, int64_t n_pairs, const acoss_simple_params *p,
+                             float *scores);
+/* Same with DEVICE buffers, asynchronous on the context's stream (no host synchronisation); acoss_sync() waits. */
+int acoss_simple_score_pairs_device(acoss_ctx *ctx, const int32_t *pairs_dev, int64_t n_pairs,
+                                    const acoss_simple_params *p, float *scores_dev);
+/* Debug dump of one pair: OTI, the float64 matrix profile and its index (n_q - m + 1 entries each) and the score.
+ * Any output pointer may be NULL.  Host buffers. */
+int acoss_simple_dump_pair(acoss_ctx *ctx, int32_t q, int32_t r, const acoss_simple_params *p, int32_t *oti,
+                           double *profile, int32_t *index, float *score);
+
 /* Device milliseconds of the EarlyFusion stages since acoss_set_profiling(ctx, 1): [0] CSM contractions,
  * [1] k-NN binarisation, [2] Smith-Waterman DP, [3] getWCSM row/column radii, [4] fusion (exp) pass. */
 int acoss_ef_stage_ms(acoss_ctx *ctx, double ms[5]);
