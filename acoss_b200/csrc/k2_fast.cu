@@ -59,14 +59,16 @@ struct PairHdr {                    // per-slot header written by fast_prep_kern
     float kf[2];                    // fractional rank (float32, essentia arithmetic)
     int32_t lo1, sh1;               // origin of the pair's item range (fixed point) / shift of a 64-bin split of it
     int32_t hi1;                    // end of the pair's item range
-    int32_t pad;
+    int32_t dz;                     // tensor sweeps: bound on z' - z (k2_tc.inl), the low-side widening of emit's zones; else 0
 };
+
+struct TcShift { int s0, s1, s2; unsigned m0; };       // tensor sweeps (k2_tc.inl): e0, 8 - e0, 16 - e0, 2^e0
 
 struct FastLayout {
     size_t slot_bytes;
     size_t off_hdr, off_rrot, off_aaf, off_bbf, off_aai, off_bbi, off_lo, off_w, off_cb, off_sh, off_cnt,
         off_cand, off_candz, off_zin, off_zout, off_rowpack, off_pool, off_pcnt, off_samp_r, off_samp_c,
-        off_lsel, off_wlist, off_wcnt, off_win, off_qpl, off_rpl, off_tcq;
+        off_lsel, off_wlist, off_wcnt, off_win, off_qpl, off_rpl, off_lsum, off_tcq;
     int max_rows, max_cols, max_frames, lines, pool_cap;
     int plane_frames;                   // frames per byte plane of the tensor sweeps (zero padded past the track end)
     int slog;                           // log2 of the diagonal sampling stride S
@@ -130,6 +132,7 @@ FastLayout make_layout(const SlotGeom &g, int max_frames) {
     L.plane_frames = max_frames + TC_PAD + 16;
     L.off_qpl = take((size_t)3 * L.plane_frames * 16);          // query byte planes [h, l1, l2][frame][16]
     L.off_rpl = take((size_t)3 * L.plane_frames * 16);          // rotated reference byte planes
+    L.off_lsum = take((size_t)2 * L.plane_frames * 4);          // per frame: sum of its h bytes | sum of its l1 bytes << 16 (q, r)
     L.off_tcq = take(4 * 4);                                    // next work item of each tensor sweep (slot 0's copy serves the call)
     L.slot_bytes = align_up(o, 256);
     return L;
@@ -142,6 +145,7 @@ __device__ __forceinline__ T *slot_ptr(char *base, const FastLayout &L, int slot
 
 // Per-row parameters of the emit sweep: {aa_fix, 4 EPS - rowLo, rowW + 4 EPS, aa_fix - rowLo + 2 EPS}.  With ar = z - (rowLo - 2 EPS):
 //   ar = .w + bb - T,   row zone <=> (unsigned)ar < .z,   near zero (z < 2 EPS) <=> ar < .y,   rowLo - 2 EPS = 2 EPS - .y
+// (the tensor sweeps pass rowLo = lo - dz, rowW = w + dz: their bracket [lo, lo + w) is in z', DESIGN.md 4.2)
 __device__ __forceinline__ int4 pack_row(int aa, int lo, int w) { return make_int4(aa, 4 * EPS - lo, w + 4 * EPS, aa - lo + 2 * EPS); }
 __device__ __forceinline__ int row_lo_e(const int4 &rp) { return 2 * EPS - rp.y; }
 
@@ -197,8 +201,9 @@ __device__ __forceinline__ void load_frame(const float *__restrict__ p, float (&
 __global__ void __launch_bounds__(256) fast_prep_kernel(TrackSet ts, const int32_t *__restrict__ pairs,
                                                         const int32_t *__restrict__ oti, int64_t first,
                                                         FastLayout L, char *__restrict__ scratch, float qperc,
-                                                        int guard, float fx_scale, float q_scale) {
+                                                        int guard, float fx_scale, float q_scale, TcShift sh3) {
     __shared__ int s_max[2];
+    __shared__ int s_lmax[4];                                 // largest window sums: h of q, h of r, l1 of q, l1 of r
     const int slot = blockIdx.x;
     const int64_t k = first + slot;
     const int q = pairs[2 * k], r = pairs[2 * k + 1], s = oti[k] % NBINS;
@@ -208,12 +213,14 @@ __global__ void __launch_bounds__(256) fast_prep_kernel(TrackSet ts, const int32
     const float *R = ts.frames + ts.offsets[r] * NBINS;
     float *rrot = slot_ptr<float>(scratch, L, slot, L.off_rrot);
     if (threadIdx.x < 2) s_max[threadIdx.x] = 0;
+    if (threadIdx.x < 4) s_lmax[threadIdx.x] = 0;
     for (int idx = threadIdx.x; idx < (nr + 8) * NBINS; idx += blockDim.x) {
         const int f = idx / NBINS, b = idx - f * NBINS;
         rrot[idx] = (f < nr) ? R[f * NBINS + rot_src(b, s)] : 0.f;
     }
     // byte planes of the tensor sweeps: x_q = rint(x * 2^q_exp) < 2^24 as limbs h, l1, l2; 16-byte frames (12 bins + 4 zeros),
     // zero frames past the track end
+    uint32_t *lsum = slot_ptr<uint32_t>(scratch, L, slot, L.off_lsum);
     if (q_scale > 0.f) {
         uint4 *qpl = slot_ptr<uint4>(scratch, L, slot, L.off_qpl), *rpl = slot_ptr<uint4>(scratch, L, slot, L.off_rpl);
         for (int idx = threadIdx.x; idx < 2 * L.plane_frames; idx += blockDim.x) {
@@ -234,6 +241,10 @@ __global__ void __launch_bounds__(256) fast_prep_kernel(TrackSet ts, const int32
             uint4 *dst = isq ? qpl : rpl;
 #pragma unroll
             for (int pl = 0; pl < 3; ++pl) dst[(size_t)pl * L.plane_frames + f] = make_uint4(w[pl][0], w[pl][1], w[pl][2], 0u);
+            uint32_t sh_ = 0u, sl_ = 0u;                      // byte sums (<= 12 * 255 each)
+#pragma unroll
+            for (int c = 0; c < 3; ++c) { sh_ = __dp4a(w[0][c], 0x01010101u, sh_); sl_ = __dp4a(w[1][c], 0x01010101u, sl_); }
+            lsum[idx] = sh_ | (sl_ << 16);
         }
     }
     uint32_t *cnt = slot_ptr<uint32_t>(scratch, L, slot, L.off_cnt);
@@ -262,7 +273,25 @@ __global__ void __launch_bounds__(256) fast_prep_kernel(TrackSet ts, const int32
     for (int i = Nx + threadIdx.x; i < L.max_cols + TC_PAD; i += blockDim.x) bbi[i] = TC_HUGE;
     atomicMax(&s_max[0], mxa);
     atomicMax(&s_max[1], mxb);
+    // the bound dz on z' - z of the tensor sweeps (k2_tc.inl): acc2 = l1.l1 + h.l2 + l2.h <= 255 (sum h_X + sum h_Y +
+    // min(sum l1_X, sum l1_Y)) over the 108 bytes of the two windows, z' - z <= (acc2 >> (16 - e0)) + 1 (DESIGN.md 4.2)
+    if (q_scale > 0.f) {
+        int m[4] = {0, 0, 0, 0};
+        for (int i = threadIdx.x; i < Mx + Nx; i += blockDim.x) {
+            const bool isq = i < Mx;
+            const uint32_t *src = lsum + (isq ? i : L.plane_frames + i - Mx);
+            uint32_t acc = 0u;                                // (h sum, l1 sum) of the window, no carry between the halves
+#pragma unroll
+            for (int t = 0; t < M9; ++t) acc += src[t];
+            const int sh_ = (int)(acc & 0xffffu), sl_ = (int)(acc >> 16);
+            if (isq) { m[0] = max(m[0], sh_); m[2] = max(m[2], sl_); }
+            else { m[1] = max(m[1], sh_); m[3] = max(m[3], sl_); }
+        }
+#pragma unroll
+        for (int c = 0; c < 4; ++c) atomicMax(&s_lmax[c], m[c]);
+    }
     __syncthreads();
+    const int dz = q_scale > 0.f ? ((255 * (s_lmax[0] + s_lmax[1] + min(s_lmax[2], s_lmax[3]))) >> sh3.s2) + 1 : 0;
     PairHdr *h = slot_ptr<PairHdr>(scratch, L, slot, L.off_hdr);
     int lo1 = -2 * EPS, sh1 = 0;
     const long long range1 = (long long)s_max[0] + s_max[1] + 4 * EPS + 1;
@@ -280,6 +309,7 @@ __global__ void __launch_bounds__(256) fast_prep_kernel(TrackSet ts, const int32
         h->nq = nq; h->nr = nr; h->Mx = Mx; h->Nx = Nx;
         for (int o = 0; o < 2; ++o) { h->fk[o] = fk2[o]; h->ck[o] = ck2[o]; h->quirk[o] = quirk2[o]; h->kf[o] = kf2[o]; }
         h->lo1 = lo1; h->sh1 = sh1; h->hi1 = lo1 + (int)range1;
+        h->dz = dz;
     }
     // level-1 bracket state for every line; emit-ready defaults for quirk sides (threshold 0)
     int32_t *lo = slot_ptr<int32_t>(scratch, L, slot, L.off_lo), *w = slot_ptr<int32_t>(scratch, L, slot, L.off_w);
@@ -1105,18 +1135,27 @@ __global__ void __launch_bounds__(32 * WPC, MINB) fast_emit_kernel(TrackSet ts, 
 }
 
 // ------------------------------------------------------------------------------------------------
-// scatter: the pair's pool of uncertain cells -> per-row / per-column candidate lists (index + fixed-point item)
+// scatter: the pair's pool of uncertain cells -> per-row / per-column candidate lists (index + fixed-point item).  A
+// candidate is flagged "below" when it lies below its line's bracket in the item the histogram levels counted: z (FFMA2
+// sweeps) or z' (tensor sweeps, z <= z' <= z + dz).  With ar = z - (lo - dz - 2 EPS): below for ar < 2 EPS, not below for
+// ar >= dz + 2 EPS; the cells in between (the band, tensor sweeps only) are queued and their z' recomputed from the byte
+// planes once the CTA's records are placed.
 // ------------------------------------------------------------------------------------------------
 constexpr int SCAT_CHUNK = 4096;    // pool records per CTA
 
-__global__ void __launch_bounds__(256) fast_scatter_kernel(int n, FastLayout L, char *__restrict__ scratch,
-                                                           int64_t first, uint32_t *__restrict__ status,
+__global__ void __launch_bounds__(256, 4) fast_scatter_kernel(int n, FastLayout L, char *__restrict__ scratch,
+                                                           int64_t first, TcShift sh3, uint32_t *__restrict__ status,
                                                            uint32_t *__restrict__ dbg) {
+    __shared__ uint32_t s_band[SCAT_CHUNK];                   // record - e0 | row slot << 12 | column slot << 20 (0xff: none)
+    __shared__ int s_nband;
     const int slot = blockIdx.y;
     if (slot >= n) return;
     const uint32_t cntv = *slot_ptr<uint32_t>(scratch, L, slot, L.off_pcnt);
     const uint32_t e0 = blockIdx.x * SCAT_CHUNK;
     if (e0 >= cntv && blockIdx.x) return;
+    if (threadIdx.x == 0) s_nband = 0;
+    __syncthreads();
+    const int dz = slot_ptr<PairHdr>(scratch, L, slot, L.off_hdr)->dz;
     if (cntv > (uint32_t)L.pool_cap && blockIdx.x == 0 && threadIdx.x == 0)
         atomicOr(&status[first + slot], PAIR_ST_FALLBACK | 16u);          // reason 16: pool overflow
     const uint32_t m = min(min(cntv, (uint32_t)L.pool_cap), e0 + SCAT_CHUNK);
@@ -1132,7 +1171,7 @@ __global__ void __launch_bounds__(256) fast_scatter_kernel(int n, FastLayout L, 
     for (uint32_t eb = e0 + threadIdx.x; eb < m; eb += SU * blockDim.x) {
         int ii[SU], jj[SU], zz_[SU];
         unsigned pr[SU], pc[SU];
-        bool rz[SU], cz[SU], lowr[SU], lowc[SU];
+        bool rz[SU], cz[SU], lowr[SU], lowc[SU], bandr[SU], bandc[SU];
 #pragma unroll
         for (int u = 0; u < SU; ++u) {
             const uint32_t e = eb + u * blockDim.x;
@@ -1141,11 +1180,13 @@ __global__ void __launch_bounds__(256) fast_scatter_kernel(int n, FastLayout L, 
                 const uint2 rec = pool[e];
                 const int i = rec.x & 0x3fff, j = (rec.x >> 14) & 0x3fff;
                 const int4 rp = rowpack[i];                   // pack_row(..)
-                const int ar = (int)rec.y, z = ar + row_lo_e(rp), ac = z - (lo_c[j] - 2 * EPS);   // the record carries ar = z - (rowLo - 2 EPS)
+                const int ar = (int)rec.y, z = ar + row_lo_e(rp), ac = z - (lo_c[j] - dz - 2 * EPS);   // the record carries ar = z - (rowLo - 2 EPS)
                 const bool zz = z < 2 * EPS;                  // near-zero item: always evaluated exactly
                 rz[u] = (ar >= 0 && ar < rp.z) || zz;
-                cz[u] = ac >= 0 && ac < w_c[j] + 4 * EPS;
+                cz[u] = ac >= 0 && ac < w_c[j] + dz + 4 * EPS;
                 lowr[u] = ar < 2 * EPS; lowc[u] = ac < 2 * EPS;
+                bandr[u] = rz[u] && !lowr[u] && ar < dz + 2 * EPS;
+                bandc[u] = cz[u] && !lowc[u] && ac < dz + 2 * EPS;
                 ii[u] = i; jj[u] = j; zz_[u] = z;
             }
         }
@@ -1156,16 +1197,37 @@ __global__ void __launch_bounds__(256) fast_scatter_kernel(int n, FastLayout L, 
         }
 #pragma unroll
         for (int u = 0; u < SU; ++u) {
-            if (rz[u] && pr[u] < CAND_CAP) {
+            const bool wr = rz[u] && pr[u] < CAND_CAP, wc = cz[u] && pc[u] < CAND_CAP;
+            if (wr) {
                 cand[(size_t)ii[u] * CAND_CAP + pr[u]] = (uint16_t)(jj[u] | (lowr[u] ? 0x8000 : 0));
                 candz[(size_t)ii[u] * CAND_CAP + pr[u]] = zz_[u];
             }
-            if (cz[u] && pc[u] < CAND_CAP) {
+            if (wc) {
                 const size_t line = (size_t)(L.max_rows + jj[u]);
                 cand[line * CAND_CAP + pc[u]] = (uint16_t)(ii[u] | (lowc[u] ? 0x8000 : 0));
                 candz[line * CAND_CAP + pc[u]] = zz_[u];
             }
+            const bool br = wr && bandr[u], bc = wc && bandc[u];
+            if (br || bc)
+                s_band[atomicAdd(&s_nband, 1)] = (eb + u * blockDim.x - e0) | ((br ? pr[u] : 0xffu) << 12) | ((bc ? pc[u] : 0xffu) << 20);
         }
+    }
+    __syncthreads();
+    // the band: z' of the cell (k2_tc.inl: tc_coarse_T), below iff z' < lo  <=>  ar + (z' - z) < dz + 2 EPS
+    const int nb = s_nband;
+    if (nb) {
+        const uint4 *qpl = slot_ptr<uint4>(scratch, L, slot, L.off_qpl), *rpl = slot_ptr<uint4>(scratch, L, slot, L.off_rpl);
+        const int32_t *aai = slot_ptr<int32_t>(scratch, L, slot, L.off_aai), *bbi = slot_ptr<int32_t>(scratch, L, slot, L.off_bbi);
+        for (int t = threadIdx.x; t < nb; t += blockDim.x) {
+            const uint32_t q = s_band[t], pr1 = (q >> 12) & 0xffu, pc1 = q >> 20;
+            const uint2 rec = pool[e0 + (q & 0xfffu)];
+            const int i = rec.x & 0x3fff, j = (rec.x >> 14) & 0x3fff;
+            const int ar = (int)rec.y, z = ar + row_lo_e(rowpack[i]), ac = z - (lo_c[j] - dz - 2 * EPS);
+            const int d = aai[i] + bbi[j] - tc_coarse_T(qpl, rpl, L.plane_frames, i, j, sh3) - z;
+            if (pr1 != 0xffu && ar + d < dz + 2 * EPS) cand[(size_t)i * CAND_CAP + pr1] |= 0x8000;
+            if (pc1 != 0xffu && ac + d < dz + 2 * EPS) cand[(size_t)(L.max_rows + j) * CAND_CAP + pc1] |= 0x8000;
+        }
+        if (threadIdx.x == 0) atomicAdd(&dbg[26], (unsigned)nb);
     }
     if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&dbg[24], min(cntv, (uint32_t)L.pool_cap));
 }
@@ -1409,8 +1471,8 @@ __global__ void __launch_bounds__(128) fast_thr_kernel(int64_t first, int n, Fas
             const double zi = floor(t2 / unit) - (double)EPS - 1.0, zo = ceil(t2 * (1.0 + 4.76837158203125e-07) / unit) + (double)EPS + 1.0;
             zin = (int)fmax(fmin(zi, 1.0e9), -1.0e9);
             zout = (int)fmax(fmin(zo, 1.0e9), -1.0e9);
-            // every cell the sweep emitted as certainly-in has z < lo - 2 EPS, every cell it dropped has z >= lo + w + 2 EPS
-            if (zin < lo - 2 * EPS - 1 || zout > lo + w + 2 * EPS) bad |= 1024u;   // reason 1024: threshold not between the certain sets
+            // every cell the sweep emitted as certainly-in has z < lo - dz - 2 EPS, every cell it dropped has z >= lo + w + 2 EPS
+            if (zin < lo - h->dz - 2 * EPS - 1 || zout > lo + w + 2 * EPS) bad |= 1024u;   // reason 1024: threshold not between the certain sets
         }
     }
     if (bad) atomicOr(&status[k], PAIR_ST_FALLBACK | bad);
@@ -1526,7 +1588,10 @@ int launch_k2_fast(const TrackSet &ts, const int32_t *pairs, const int32_t *oti,
     if (sweeps_env && sweeps_env[0] == 't') use_tc = ts.q_exp >= 0;
     if (sweeps_env && sweeps_env[0] == 'f') use_tc = false;
     const float q_scale = use_tc ? ldexpf(1.f, ts.q_exp) : 0.f;
-    fast_prep_kernel<<<n, 256, 0, st>>>(ts, pairs, oti, first, L, base, qperc, p.integer_guard, fx_scale, q_scale);
+    // tensor sweeps: the limb products weigh 2^e0, 2^(e0 - 8), 2^(e0 - 16) fixed-point units (k2_tc.inl), 0 <= e0 <= 6
+    const int e0 = 56 - 2 * ts.q_exp - ts.fx_exp;
+    const TcShift sh3 = use_tc ? TcShift{e0, 8 - e0, 16 - e0, 1u << e0} : TcShift{0, 0, 0, 0u};
+    fast_prep_kernel<<<n, 256, 0, st>>>(ts, pairs, oti, first, L, base, qperc, p.integer_guard, fx_scale, q_scale, sh3);
     CUDA_TRY(cudaGetLastError());
     te(K2K_PREP);
     const int outw = Sweep<RC>::OUTW, houtw = Sweep<HRC>::OUTW;
@@ -1566,12 +1631,10 @@ int launch_k2_fast(const TrackSet &ts, const int32_t *pairs, const int32_t *oti,
     // every line still live to the sparse refinement
     if (use_tc) {
         // tensor sweeps (k2_tc.inl): one CTA = 128 owned lines; items from tcgen05.mma.kind::i8 over the byte planes
-        const int e0 = 56 - 2 * ts.q_exp - ts.fx_exp;
-        const TcShift sh3 = {e0, 8 - e0, 16 - e0, 1u << e0};
         const int tstrips_c = (g.max_cols + 127) / 128, tstrips_r = (g.max_rows + 127) / 128;
         // (one CTA per SM: it holds all 512 TMEM columns; the requested shared memory keeps a second one off the SM)
-        const size_t smem_h = std::max(sizeof(TcSmem) + (size_t)(NBIN + 2) * 128 * 4, (size_t)120 * 1024);
-        const size_t smem_e = std::max(sizeof(TcSmem) + (size_t)(TC_CONS / 32) * (TC_STAGE * 32 * 8 + 64), (size_t)120 * 1024);
+        const size_t smem_h = std::max(sizeof(TcSmem<TC_NP_HIST>) + (size_t)(NBIN + 2) * 128 * 4, (size_t)120 * 1024);
+        const size_t smem_e = std::max(sizeof(TcSmem<TC_NP_EMIT>) + (size_t)(TC_CONS / 32) * (TC_STAGE * 32 * 8 + 64), (size_t)120 * 1024);
         static bool tc_attr_done[64] = {false};
         if (!tc_attr_done[dev & 63]) {
             CUDA_TRY(cudaFuncSetAttribute(tc_hist_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_h));
@@ -1638,7 +1701,7 @@ int launch_k2_fast(const TrackSet &ts, const int32_t *pairs, const int32_t *oti,
     }
     }
     tb(K2K_SCATTER);
-    fast_scatter_kernel<<<dim3((L.pool_cap + SCAT_CHUNK - 1) / SCAT_CHUNK, n), 256, 0, st>>>(n, L, base, first, status, dbg);
+    fast_scatter_kernel<<<dim3((L.pool_cap + SCAT_CHUNK - 1) / SCAT_CHUNK, n), 256, 0, st>>>(n, L, base, first, sh3, status, dbg);
     CUDA_TRY(cudaGetLastError());
     te(K2K_SCATTER);
     tb(K2K_THR);

@@ -227,13 +227,13 @@ class Engine:
     def debug_counters(self) -> dict:
         """Diagnostic counters of the last scoring call (acoss_debug_counters): dense histogram level per
         orientation (strips, live lines, bracket misses, lines left), sparse refinement (warps, sweeps,
-        lines left), listed uncertain cells, exact candidates."""
+        lines left), listed uncertain cells, exact candidates, band cells whose coarse item was recomputed."""
         d = np.zeros(32, dtype=np.int64)
         check(self._lib.acoss_debug_counters(self._ctx, d.ctypes.data))
         lv = {"col_dense": tuple(int(x) for x in d[0:4]), "row_dense": tuple(int(x) for x in d[4:8]),
               "sparse": tuple(int(x) for x in d[8:11]),
               "col_dense2": tuple(int(x) for x in d[12:16]), "row_dense2": tuple(int(x) for x in d[16:20])}
-        lv["uncertain_cells"] = int(d[24]); lv["exact_candidates"] = int(d[25])
+        lv["uncertain_cells"] = int(d[24]); lv["exact_candidates"] = int(d[25]); lv["band_cells"] = int(d[26])
         return lv
 
     def last_stats(self) -> dict:

@@ -235,7 +235,8 @@ int acoss_last_stats(acoss_ctx *ctx, int64_t stats[8]);
  * ranks fell outside the sampled bracket, lines handed to the sparse refinement.  Sparse refinement
  * out[8..10]: warps, sweeps, lines still crowded at the end.  out[12..15] / out[16..19]: the same four
  * counters for the second (gated) dense level, columns / rows.  out[24] uncertain cells the emit sweep
- * listed, out[25] candidate cells evaluated exactly. */
+ * listed, out[25] candidate cells evaluated exactly, out[26] listed cells whose coarse item the scatter kernel recomputed
+ * (tensor-core sweeps: cells within dz below a line's bracket). */
 int acoss_debug_counters(acoss_ctx *ctx, int64_t out[32]);
 
 /* Per-stage device timing of the pair pipeline, measured with CUDA events on the context stream:
