@@ -78,7 +78,12 @@ SIGNATURES = {
     "acoss_simple_score_pairs": (C.c_int, [_vp, _i32p, C.c_int64, C.POINTER(SimpleParams), _fp]),
     "acoss_simple_score_pairs_device": (C.c_int, [_vp, _i32p, C.c_int64, C.POINTER(SimpleParams), _fp]),
     "acoss_simple_dump_pair": (C.c_int, [_vp, C.c_int32, C.c_int32, C.POINTER(SimpleParams), _i32p, _vp, _i32p, _fp]),
+    "acoss_snf": (C.c_int, [_vp, _vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_double, C.c_int32,
+                            _vp, _fp, _fp, _i32p, _fp]),
+    "acoss_snf_stage_ms": (C.c_int, [_vp, _vp]),
 }
+
+SNF_MAX_K, SNF_MAX_MATS = 63, 16     # ACOSS_SNF_MAX_K, ACOSS_SNF_MAX_MATS
 
 
 def load():

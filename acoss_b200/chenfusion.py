@@ -6,14 +6,15 @@ builds ONE binary cross-recurrence plot per pair on the GPU (K1 OTI -> K2 CRP, s
 where the reference calls essentia three times per pair (latefusion_chen.py:63-73).
 
 ``do_late_fusion`` is the reference's N x N similarity-network fusion of the two finished score
-matrices (acoss/algorithms/utils/similarity_fusion.py) — post-processing outside the pairwise hot
-path (SURVEY.md §2 row 8).  It is delegated to the reference's own function when the ``acoss``
-package is importable and refused otherwise.
+matrices (acoss/algorithms/utils/similarity_fusion.py).  By default it is delegated to the reference's
+own function when the ``acoss`` package is importable and refused otherwise; ``impl="gpu"`` runs it on
+the GPU (``acoss_b200.fusion``, k7_snf.cu).
 """
 from __future__ import annotations
 
 import numpy as np
 
+from .engine import Engine
 from .serra09 import Serra09
 
 __all__ = ["ChenFusion"]
@@ -45,15 +46,25 @@ class ChenFusion(Serra09):
             with np.errstate(divide="ignore"):
                 self.Ds[key][:, :] = (fac[None, :] / D).astype(np.float32)
 
-    def do_late_fusion(self):
-        """latefusion_chen.py:87-91 — SNF of the two distance matrices, then the sign flip."""
-        try:
-            from acoss.algorithms.utils.similarity_fusion import doSimilarityFusion
-        except Exception as e:  # the reference package (and its heavy imports) is not installed
-            raise NotImplementedError(
-                "do_late_fusion is the reference's N x N similarity-network fusion (similarity_fusion.py), "
-                "outside the pairwise hot path; install the reference package to use it") from e
-        DLate = doSimilarityFusion([self.Ds[s] for s in self.Ds], K=20, niters=20, reg_diag=1)[1]
+    def do_late_fusion(self, impl="reference"):
+        """latefusion_chen.py:87-91 — SNF of the two distance matrices, then the sign flip.  impl="reference" calls the
+        reference's doSimilarityFusion (NotImplementedError when the acoss package is not importable); impl="gpu"
+        runs the fusion on this plugin's GPU (acoss_b200.fusion) with the same keys, signs and dtypes."""
+        if impl == "gpu":
+            from .fusion import fuse
+            if self._engine is None:             # the fusion needs a device, not the resident tracks of engine()
+                self._engine = Engine(self.device)
+            DLate = fuse([self.Ds[s] for s in self.Ds], K=20, niters=20, reg_diag=1, engine=self._engine)["fused"]
+        elif impl == "reference":
+            try:
+                from acoss.algorithms.utils.similarity_fusion import doSimilarityFusion
+            except Exception as e:  # the reference package (and its heavy imports) is not installed
+                raise NotImplementedError(
+                    "do_late_fusion is the reference's N x N similarity-network fusion (similarity_fusion.py); "
+                    "install the reference package to use it, or pass impl='gpu'") from e
+            DLate = doSimilarityFusion([self.Ds[s] for s in self.Ds], K=20, niters=20, reg_diag=1)[1]
+        else:
+            raise ValueError("impl must be 'reference' or 'gpu', got %r" % (impl,))
         for key in self.Ds:
             self.Ds[key] *= -1                    # switch back to larger scores being closer
         self.Ds["Late"] = DLate

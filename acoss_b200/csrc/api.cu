@@ -70,7 +70,7 @@ struct acoss_ctx {
     size_t ev_used = 0;
     struct Span { int stage; cudaEvent_t a, b; };
     std::vector<Span> spans;
-    double stage_ms[32] = {0};   // [0..3] Serra09 pipeline, [4..8] EarlyFusion pipeline, [16 + K2K_*] K2 kernels
+    double stage_ms[32] = {0};   // [0..3] Serra09 pipeline, [4..8] EarlyFusion pipeline, [9..12] SNF, [16 + K2K_*] K2 kernels
     // EarlyFusion block features (acoss_ef_set_tracks): float64, row pitch ef_dp[k], kinds mfccs / ssms / chromas
     Buf ef_feat[3], ef_sq[2], ef_cmed, ef_off;
     std::vector<int64_t> ef_hoff;
@@ -90,12 +90,13 @@ static cudaEvent_t get_event(acoss_ctx *c) {
     }
     return c->ev_pool[c->ev_used++];
 }
-static const char *const STAGE_NAMES[9] = {"acoss/K1 oti", "acoss/K2 crp", "acoss/K3 dp", "acoss/K2 emit", "acoss/EF csm", "acoss/EF knn",
-                                           "acoss/EF sw", "acoss/EF radii", "acoss/EF fuse"};
+static const char *const STAGE_NAMES[13] = {"acoss/K1 oti", "acoss/K2 crp", "acoss/K3 dp", "acoss/K2 emit", "acoss/EF csm", "acoss/EF knn",
+                                            "acoss/EF sw", "acoss/EF radii", "acoss/EF fuse", "acoss/SNF h2d", "acoss/SNF affinity",
+                                            "acoss/SNF diffusion", "acoss/SNF average"};
 struct StageTimer {     // NVTX range around a pipeline stage (host side: the enqueue); CUDA events [a, b] when profiling is on
     acoss_ctx *c; int stage; cudaEvent_t a = nullptr; bool open = true;
     StageTimer(acoss_ctx *c_, int s) : c(c_), stage(s) {
-        nvtxRangePushA(STAGE_NAMES[s < 9 ? s : 1]);
+        nvtxRangePushA(STAGE_NAMES[s < 13 ? s : 1]);
         if (c->profiling) { a = get_event(c); cudaEventRecord(a, c->stream); }
     }
     void stop() {
@@ -1232,6 +1233,104 @@ int acoss_simple_dump_pair(acoss_ctx *c, int32_t q, int32_t r, const acoss_simpl
     if (oti) CUDA_TRY(cudaMemcpyAsync(oti, c->sp_oti.p, 4, cudaMemcpyDeviceToHost, c->stream));
     if (score) CUDA_TRY(cudaMemcpyAsync(score, c->sp_scores.p, 4, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
+    return ACOSS_OK;
+}
+
+
+// ---- Similarity-network fusion (k7_snf.cu) -----------------------------------------------------------------------
+
+int acoss_snf(acoss_ctx *c, const float *const *D, int32_t n_mats, int32_t n, int32_t K, int32_t niters, double reg_diag,
+              double reg_neighbs, int32_t jacobi, double *fused, float *W, float *P, int32_t *S_idx, float *S_val) {
+    if (!c || !D || !fused) { acoss_set_error("snf: NULL argument"); return ACOSS_E_INVALID; }
+    if (n_mats < 2 || n_mats > ACOSS_SNF_MAX_MATS) {
+        acoss_set_error("snf: %d score matrices; 2..%d supported (the reference divides by n_mats - 1)", n_mats, ACOSS_SNF_MAX_MATS);
+        return ACOSS_E_INVALID;
+    }
+    for (int m = 0; m < n_mats; ++m)
+        if (!D[m]) { acoss_set_error("snf: score matrix %d is NULL", m); return ACOSS_E_INVALID; }
+    if (K < 1 || K > ACOSS_SNF_MAX_K) { acoss_set_error("snf: K = %d outside 1..%d", K, ACOSS_SNF_MAX_K); return ACOSS_E_INVALID; }
+    if (n < 2 || n > 65535 || K + 1 >= n) {
+        acoss_set_error("snf: n = %d with K = %d; K + 1 < n <= 65535 required (np.partition raises for kth >= n)", n, K);
+        return ACOSS_E_INVALID;
+    }
+    if (niters < 0) { acoss_set_error("snf: niters = %d < 0", niters); return ACOSS_E_INVALID; }
+    CUDA_TRY(cudaSetDevice(c->device));
+    cudaStream_t st = c->stream;
+    const int64_t N2 = (int64_t)n * n;
+    const int sets = niters == 0 ? 0 : (jacobi ? 2 : 1);     // float64 Pts sets: Jacobi keeps the previous iteration
+    const std::vector<int32_t> leaves = snf_leaf_offsets(n);
+    auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    const size_t b_p = up((size_t)n_mats * N2 * 4), b_s = up((size_t)n_mats * n * K * 4), b_pts = up((size_t)sets * n_mats * N2 * 8),
+                 b_x = up((size_t)N2 * 8), b_t = niters ? up((size_t)N2 * 8) : 0, b_md = up((size_t)n * 4), b_leaf = up(leaves.size() * 4);
+    const size_t total = b_p + 2 * b_s + b_pts + b_x + b_t + b_md + b_leaf;
+    if ((int64_t)total > c->ws_limit) {
+        acoss_set_error("snf: %zu bytes of device workspace needed, limit %lld (acoss_set_workspace_limit)", total, (long long)c->ws_limit);
+        return ACOSS_E_NOMEM;
+    }
+    struct Scratch { void *p = nullptr; ~Scratch() { if (p) cudaFree(p); } } ws;   // released when the call returns
+    if (cudaMalloc(&ws.p, total) != cudaSuccess) {
+        cudaGetLastError();
+        ws.p = nullptr;
+        acoss_set_error("snf: cudaMalloc(%zu bytes) failed", total);
+        return ACOSS_E_NOMEM;
+    }
+    char *p = (char *)ws.p;
+    float *dP = (float *)p; p += b_p;                          // P of every matrix (the first iteration's Pts)
+    int32_t *dSi = (int32_t *)p; p += b_s;
+    float *dSv = (float *)p; p += b_s;
+    double *dPts = (double *)p; p += b_pts;                    // [set][matrix] float64 Pts
+    double *dX = (double *)p; p += b_x;                        // X^T; the score staging + DSym / W before; fused after
+    double *dT = (double *)p; p += b_t;                        // A^T
+    float *dmd = (float *)p; p += b_md;
+    int32_t *dleaf = (int32_t *)p;
+    float *dstage = (float *)dX, *dw = (float *)dX + N2;
+    CUDA_TRY(cudaMemcpyAsync(dleaf, leaves.data(), leaves.size() * 4, cudaMemcpyHostToDevice, st));
+    for (int m = 0; m < n_mats; ++m) {
+        StageTimer h2d(c, 9);
+        CUDA_TRY(cudaMemcpyAsync(dstage, D[m], (size_t)N2 * 4, cudaMemcpyHostToDevice, st));
+        h2d.stop();
+        StageTimer aff(c, 10);
+        TRY(launch_snf_affinity(dstage, n, K, dw, dmd, dleaf, (int)leaves.size() - 1, dP + m * N2, dSi + (int64_t)m * n * K,
+                                dSv + (int64_t)m * n * K, st));
+        aff.stop();
+        if (W) CUDA_TRY(cudaMemcpyAsync(W + m * N2, dw, (size_t)N2 * 4, cudaMemcpyDeviceToHost, st));
+    }
+    if (P) CUDA_TRY(cudaMemcpyAsync(P, dP, (size_t)n_mats * N2 * 4, cudaMemcpyDeviceToHost, st));
+    if (S_idx) CUDA_TRY(cudaMemcpyAsync(S_idx, dSi, (size_t)n_mats * n * K * 4, cudaMemcpyDeviceToHost, st));
+    if (S_val) CUDA_TRY(cudaMemcpyAsync(S_val, dSv, (size_t)n_mats * n * K * 4, cudaMemcpyDeviceToHost, st));
+    // Iteration 0 reads the float32 P; later ones read set (it - 1) % sets and write set it % sets, so with one set
+    // (jacobi = 0) Pts[k < i] already hold this iteration's values
+    auto pts = [&](int set, int m) { return dPts + ((int64_t)set * n_mats + m) * N2; };
+    StageTimer dif(c, 11);
+    for (int it = 0; it < niters; ++it) {
+        for (int i = 0; i < n_mats; ++i) {
+            const void *src[ACOSS_SNF_MAX_MATS];
+            int ns = 0;
+            for (int k = 0; k < n_mats; ++k)
+                if (k != i) src[ns++] = it == 0 ? (const void *)(dP + k * N2) : (const void *)pts((it - 1) % sets, k);
+            TRY(launch_snf_mix(src, ns, it == 0, it == 0 ? nullptr : pts((it - 1) % sets, i), n, (double)(n_mats - 1), dX, st));
+            TRY(launch_snf_spmm(dX, dSi + (int64_t)i * n * K, dSv + (int64_t)i * n * K, n, K, true, 0.0, 0.0, dT, st));
+            TRY(launch_snf_spmm(dT, dSi + (int64_t)i * n * K, dSv + (int64_t)i * n * K, n, K, false, reg_diag, reg_neighbs,
+                                pts(it % sets, i), st));
+        }
+    }
+    dif.stop();
+    StageTimer fin(c, 12);
+    const void *src[ACOSS_SNF_MAX_MATS];
+    for (int m = 0; m < n_mats; ++m) src[m] = niters == 0 ? (const void *)(dP + m * N2) : (const void *)pts((niters - 1) % sets, m);
+    TRY(launch_snf_average(src, n_mats, niters == 0, N2, dX, st));
+    CUDA_TRY(cudaMemcpyAsync(fused, dX, (size_t)N2 * 8, cudaMemcpyDeviceToHost, st));
+    fin.stop();
+    CUDA_TRY(cudaStreamSynchronize(st));
+    return ACOSS_OK;
+}
+
+int acoss_snf_stage_ms(acoss_ctx *c, double ms[4]) {
+    if (!c || !ms) { acoss_set_error("snf_stage_ms: NULL argument"); return ACOSS_E_INVALID; }
+    CUDA_TRY(cudaSetDevice(c->device));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
+    fold_spans(c);
+    for (int i = 0; i < 4; ++i) ms[i] = c->stage_ms[9 + i];
     return ACOSS_OK;
 }
 

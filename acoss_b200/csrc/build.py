@@ -4,7 +4,7 @@ import subprocess
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-SOURCES = ["api.cu", "k0_onramp.cu", "k1_oti.cu", "k2_exact.cu", "k2_fast.cu", "k3_dp.cu", "k4_knn.cu", "k5_earlyfusion.cu", "k6_simple.cu"]
+SOURCES = ["api.cu", "k0_onramp.cu", "k1_oti.cu", "k2_exact.cu", "k2_fast.cu", "k3_dp.cu", "k4_knn.cu", "k5_earlyfusion.cu", "k6_simple.cu", "k7_snf.cu"]
 HEADERS = ["common.cuh", "k2_fast.cuh", "k2_tc.inl", "../../include/acoss_b200.h"]
 OUT = os.path.join(HERE, "libacoss_b200.so")
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

@@ -4,6 +4,8 @@
 #include <stdint.h>
 #include <stdio.h>
 
+#include <vector>
+
 #include "../../include/acoss_b200.h"
 
 #define NBINS ACOSS_NBINS
@@ -183,3 +185,15 @@ int launch_ef_linestat(const double *csm, int64_t kind_stride, int64_t slot_elem
 int launch_ef_fuse(const double *csm, int64_t kind_stride, int64_t slot_elems, const int64_t *offsets,
                    const int32_t *pairs, int n, int max_rows, int max_cols, const double *stat,
                    int64_t stat_kind_stride, int stat_pitch, double *out, cudaStream_t st);
+
+// K7: similarity-network fusion (k7_snf.cu).  Leaf boundaries of numpy's pairwise sum over n elements (n_leaves + 1
+// entries); the affinity stages of one matrix (d: the scores, dw: DSym, then W, in place; md: MeanDist); one diffusion
+// input written transposed; S . Y (transposed output, or the regularised row-major one); the final average.
+std::vector<int32_t> snf_leaf_offsets(int n);
+int launch_snf_affinity(const float *d, int n, int K, float *dw, float *md, const int32_t *leaf_off, int n_leaves,
+                        float *P, int32_t *s_idx, float *s_val, cudaStream_t st);
+int launch_snf_mix(const void *const *src, int nsrc, bool f32, const double *prev, int n, double den, double *xt,
+                   cudaStream_t st);
+int launch_snf_spmm(const double *Y, const int32_t *s_idx, const float *s_val, int n, int K, bool transposed,
+                    double reg_diag, double reg_neighbs, double *out, cudaStream_t st);
+int launch_snf_average(const void *const *src, int nsrc, bool f32, int64_t cells, double *out, cudaStream_t st);

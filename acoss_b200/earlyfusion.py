@@ -14,7 +14,8 @@ on-ramp of ``load_features`` (madmom onsets, skimage resize — absent from this
 therefore returns precomputed block features exactly as the reference's returns them (keys 'mfccs', 'ssms',
 'chromas', 'chroma_med', 'label'), from memory or from the reference's own cache file layout.
 ``do_late_fusion`` (N x N similarity-network fusion of finished score matrices) is delegated to the
-reference's function when the ``acoss`` package is importable.
+reference's function when the ``acoss`` package is importable; ``impl="gpu"`` runs it on the GPU
+(``acoss_b200.fusion``, k7_snf.cu).
 
 ``sw_of_csms`` scores caller-supplied float64 cross-similarity matrices on the GPU (``acoss_knn_sw``).  There is
 no host (numpy) implementation of any stage in this package: without the CUDA library every call raises.
@@ -188,15 +189,23 @@ class EarlyFusion(CoverAlgorithm):
         self._ensure_resident()
         return self.engine().ef_score_pairs(pairs.astype(np.int32), self.kappa, self.K)
 
-    def do_late_fusion(self):
-        """earlyfusion_traile.py:200-206 — SNF of the finished N x N score matrices (post-processing outside
-        the pairwise hot path): the reference's own doSimilarityFusion when importable."""
-        try:
-            from acoss.algorithms.utils.similarity_fusion import doSimilarityFusion
-        except Exception as e:
-            raise NotImplementedError(
-                "do_late_fusion is the reference's N x N similarity-network fusion (similarity_fusion.py), "
-                "outside the pairwise hot path; install the reference package to use it") from e
+    def do_late_fusion(self, impl="reference"):
+        """earlyfusion_traile.py:200-206 — SNF of the finished N x N score matrices.  impl="reference" calls the
+        reference's own doSimilarityFusion (NotImplementedError when the acoss package is not importable);
+        impl="gpu" runs both fusions on this plugin's GPU (acoss_b200.fusion) with the same keys and dtypes."""
+        if impl == "gpu":
+            from .fusion import fuse
+            def doSimilarityFusion(Scores, K, niters, reg_diag):
+                return None, fuse(Scores, K=K, niters=niters, reg_diag=reg_diag, engine=self.engine())["fused"]
+        elif impl == "reference":
+            try:
+                from acoss.algorithms.utils.similarity_fusion import doSimilarityFusion
+            except Exception as e:
+                raise NotImplementedError(
+                    "do_late_fusion is the reference's N x N similarity-network fusion (similarity_fusion.py); "
+                    "install the reference package to use it, or pass impl='gpu'") from e
+        else:
+            raise ValueError("impl must be 'reference' or 'gpu', got %r" % (impl,))
         self.Ds["late"] = doSimilarityFusion([1.0 / (1.0 + self.Ds[s]) for s in ["chromas", "ssms", "mfccs"]],
                                              K=20, niters=20, reg_diag=1)[1]
         self.Ds["early+late"] = doSimilarityFusion(

@@ -13,7 +13,7 @@ from . import _lib
 from ._lib import ALIGN_DMAX, ALIGN_DMAX_PLAIN, ALIGN_QMAX, ALIGN_SW, AcossError, Params, check, default_params  # noqa: F401
 from ._lib import SimpleParams, simple_default_params  # noqa: F401
 
-__all__ = ["Engine", "AcossError", "default_params", "pack_tracks"]
+__all__ = ["Engine", "AcossError", "default_params", "pack_tracks", "check_snf_args"]
 
 
 def pack_tracks(tracks):
@@ -28,6 +28,21 @@ def pack_tracks(tracks):
     for t, o in zip(tracks, offsets[:-1]):
         frames[o:o + t.shape[0]] = t            # handles the reference's transposed views
     return frames, offsets
+
+
+def check_snf_args(n_mats: int, n: int, K: int, niters: int = 0):
+    """The arguments acoss_snf refuses, as ValueError: n_mats outside 2..16 (the reference divides by n_mats - 1 and
+    returns NaN for one matrix), K outside 1..63, K + 1 >= n (np.partition raises ValueError), niters < 0."""
+    if not 2 <= n_mats <= _lib.SNF_MAX_MATS:
+        raise ValueError("similarity fusion needs 2..%d score matrices, got %d" % (_lib.SNF_MAX_MATS, n_mats))
+    if not 1 <= K <= _lib.SNF_MAX_K:
+        raise ValueError("K = %d outside 1..%d" % (K, _lib.SNF_MAX_K))
+    if K + 1 >= n:
+        raise ValueError("kth(=%d) out of bounds (%d): K + 1 must be smaller than the number of tracks" % (K + 1, n))
+    if n > 65535:
+        raise ValueError("n = %d tracks; at most 65535 supported" % n)
+    if niters < 0:
+        raise ValueError("niters = %d < 0" % niters)
 
 
 class Engine:
@@ -335,3 +350,35 @@ class Engine:
         st = np.zeros(4, dtype=np.int64)
         check(self._lib.acoss_ef_last_stats(self._ctx, st.ctypes.data))
         return dict(pairs=int(st[0]), cells=int(st[1]), launches=int(st[2]), chunks=int(st[3]))
+
+    # -- similarity-network fusion -------------------------------------------------------------------
+    def snf(self, Ds, K: int = 5, niters: int = 20, reg_diag: float = 1.0, reg_neighbs: float = 0.5,
+            jacobi: bool = False, want_W: bool = False, want_PS: bool = False) -> dict:
+        """doSimilarityFusion of the n x n score matrices Ds on the GPU (acoss_snf): dict(fused float64 (n, n)), plus
+        W float32 (n_mats, n, n) when want_W, and P float32 (n_mats, n, n), S_idx int32 / S_val float32
+        (n_mats, n, K) when want_PS.  jacobi is switch L1."""
+        mats = [np.ascontiguousarray(D, dtype=np.float32) for D in Ds]
+        n = int(mats[0].shape[0]) if mats else 0
+        for D in mats:
+            if D.ndim != 2 or D.shape != (n, n):
+                raise ValueError("score matrices must all be square and of one size; got %r" % (D.shape,))
+        check_snf_args(len(mats), n, int(K), int(niters))
+        ptrs = (C.c_void_p * len(mats))(*[D.ctypes.data for D in mats])
+        out = dict(fused=np.empty((n, n), dtype=np.float64))
+        if want_W:
+            out["W"] = np.empty((len(mats), n, n), dtype=np.float32)
+        if want_PS:
+            out["P"] = np.empty((len(mats), n, n), dtype=np.float32)
+            out["S_idx"] = np.empty((len(mats), n, int(K)), dtype=np.int32)
+            out["S_val"] = np.empty((len(mats), n, int(K)), dtype=np.float32)
+        ptr = lambda k: out[k].ctypes.data if k in out else None
+        check(self._lib.acoss_snf(self._ctx, ptrs, len(mats), n, int(K), int(niters), float(reg_diag),
+                                  float(reg_neighbs), int(bool(jacobi)), ptr("fused"), ptr("W"), ptr("P"),
+                                  ptr("S_idx"), ptr("S_val")))
+        return out
+
+    def snf_stage_ms(self) -> dict:
+        """Accumulated device milliseconds of the fusion stages since set_profiling(True)."""
+        ms = np.zeros(4, dtype=np.float64)
+        check(self._lib.acoss_snf_stage_ms(self._ctx, ms.ctypes.data))
+        return dict(h2d=float(ms[0]), affinity=float(ms[1]), diffusion=float(ms[2]), average_d2h=float(ms[3]))

@@ -218,6 +218,36 @@ int acoss_simple_score_pairs_device(acoss_ctx *ctx, const int32_t *pairs_dev, in
 int acoss_simple_dump_pair(acoss_ctx *ctx, int32_t q, int32_t r, const acoss_simple_params *p, int32_t *oti,
                            double *profile, int32_t *index, float *score);
 
+/* ---- Similarity-network fusion (similarity_fusion.py, doSimilarityFusion) ------------------------------------------
+ * The late fusion of ChenFusion.do_late_fusion (latefusion_chen.py:87-91: Ds["Late"]) and EarlyFusion.do_late_fusion
+ * (earlyfusion_traile.py:200-206: Ds["late"], Ds["early+late"]) over the finished N x N score matrices. */
+#define ACOSS_SNF_MAX_K 63      /* neighbours K of getS / getW (the plugins use 20)                                  */
+#define ACOSS_SNF_MAX_MATS 16   /* score matrices per fusion                                                         */
+
+/* Replaces doSimilarityFusion(D, K, niters, reg_diag, reg_neighbs) (similarity_fusion.py: getW, getP, getS,
+ * doSimilarityFusionWs).  D[m] (m < n_mats) are row-major n x n float32 host matrices; fused (n x n float64, host)
+ * receives the fused matrix.  getW: DSym = 0.5 (D + D^T) with a zero diagonal, MeanDist = mean of the K+1 smallest
+ * DSym of the row * (K+1) / K, W = exp(-DSym^2 / (2 (0.5 Eps)^2)), Eps = (MeanDist_r + MeanDist_c + DSym) / 3, in
+ * float32 and numpy's operation order (the K+1 smallest are added in ascending order).  getP: W / numpy's pairwise
+ * float32 row sum.  getS: the K largest W of each row (ties: lowest column; NaN after +inf as in np.argpartition),
+ * normalised by their sum and stored in ascending column order.  Diffusion: niters iterations of, for i in order,
+ * Pts[i] = S_i ((nextPts[i] * 0 + sum_{k != i} Pts[k]) / (n_mats - 1)) S_i^T + reg_diag I (if reg_diag > 0)
+ * + reg_neighbs on |r - c| == 1 (if reg_neighbs > 0), float64, each sparse product in stored-slot order with separate
+ * roundings (scipy csr_matvecs).  jacobi = 0 (switch L1 default) is the reference's `Pts = nextPts` aliasing: the
+ * first iteration reads the float32 P of every matrix, later ones read the Pts[k] already updated in the same
+ * iteration for k < i; jacobi = 1 reads the previous iteration's Pts for every k.  fused = (sum of Pts) / n_mats.
+ * W (n_mats x n x n float32), P (same), S_idx (n_mats x n x K int32) and S_val (same, float32) may be NULL; they
+ * receive the affinities, the transition matrices and the neighbour lists.  ACOSS_E_INVALID for n_mats outside
+ * 2..ACOSS_SNF_MAX_MATS (the reference divides by n_mats - 1 and returns NaN for one matrix), K outside
+ * 1..ACOSS_SNF_MAX_K, K + 1 >= n (np.partition raises), n > 65535 or niters < 0; ACOSS_E_NOMEM when the device
+ * workspace, n_mats n^2 (4 + 8 * (1 + jacobi)) + 16 n^2 bytes, exceeds the workspace limit.  Host buffers. */
+int acoss_snf(acoss_ctx *ctx, const float *const *D, int32_t n_mats, int32_t n, int32_t K, int32_t niters,
+              double reg_diag, double reg_neighbs, int32_t jacobi, double *fused, float *W, float *P, int32_t *S_idx,
+              float *S_val);
+/* Device milliseconds of the fusion stages since acoss_set_profiling(ctx, 1): [0] H2D of the score matrices,
+ * [1] affinity (DSym, W, P, S), [2] diffusion, [3] the final average and the D2H of the fused matrix. */
+int acoss_snf_stage_ms(acoss_ctx *ctx, double ms[4]);
+
 /* Device milliseconds of the EarlyFusion stages since acoss_set_profiling(ctx, 1): [0] CSM contractions,
  * [1] k-NN binarisation, [2] Smith-Waterman DP, [3] getWCSM row/column radii, [4] fusion (exp) pass. */
 int acoss_ef_stage_ms(acoss_ctx *ctx, double ms[5]);
