@@ -57,6 +57,7 @@ SIGNATURES = {
     "acoss_score_pairs": (C.c_int, [_vp, _i32p, C.c_int64, C.POINTER(Params), _fp]),
     "acoss_score_pairs_device": (C.c_int, [_vp, _i32p, C.c_int64, C.POINTER(Params), _fp]),
     "acoss_score_pairs_chen": (C.c_int, [_vp, _i32p, C.c_int64, C.POINTER(Params), _fp, _fp]),
+    "acoss_score_pairs_chen_device": (C.c_int, [_vp, _i32p, C.c_int64, C.POINTER(Params), _fp, _fp]),
     "acoss_sync": (C.c_int, [_vp]),
     "acoss_stream": (C.c_void_p, [_vp]),
     "acoss_oti_pairs": (C.c_int, [_vp, _i32p, C.c_int64, C.c_int32, _i32p]),

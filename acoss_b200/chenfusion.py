@@ -27,13 +27,20 @@ class ChenFusion(Serra09):
                          kappa=kappa, tau=tau, m=m, downsample_fac=downsample_fac,
                          _name="LateFusionChen", _similarity_types=("qmax", "dmax"), **kw)
 
+    def score_pairs(self, pairs):
+        """pairs (n, 2) int -> float32 (2, n): the Qmax and Dmax rows, in Ds key order, of one batched GPU call.
+        The scoring hook of all_pairwise_distributed; there is no pair_weights, so the distributed run keeps the
+        list-free triangle shard of Serra09."""
+        pairs = np.asarray(pairs).reshape(-1, 2).astype(np.int32)
+        return np.stack(self.engine().score_pairs_chen(pairs, self.params()))
+
     def similarity(self, idxs):
         """Ds["qmax"][i, j], Ds["dmax"][i, j] for every (query i, reference j) row of idxs
         (latefusion_chen.py:58-73), one batched GPU call."""
         idxs = np.asarray(idxs).reshape(-1, 2)
         if len(idxs) == 0:
             return
-        qmax, dmax = self.engine().score_pairs_chen(idxs.astype(np.int32), self.params())
+        qmax, dmax = self.score_pairs(idxs)
         self.Ds["qmax"][idxs[:, 0], idxs[:, 1]] = qmax
         self.Ds["dmax"][idxs[:, 0], idxs[:, 1]] = dmax
 

@@ -713,7 +713,7 @@ int acoss_score_pairs(acoss_ctx *c, const int32_t *pairs, int64_t K, const acoss
 
 int acoss_score_pairs_chen(acoss_ctx *c, const int32_t *pairs, int64_t K, const acoss_params *p, float *qmax_scores,
                            float *dmax_scores) {
-    if (!c || (K > 0 && (!pairs || !qmax_scores || !dmax_scores))) { acoss_set_error("score_pairs_chen: NULL argument"); return ACOSS_E_INVALID; }
+    if (!c || (K > 0 && (!pairs || !p || !qmax_scores || !dmax_scores))) { acoss_set_error("score_pairs_chen: NULL argument"); return ACOSS_E_INVALID; }
     if (K <= 0) return check_params(c, p);
     for (int64_t k = 0; k < 2 * K; ++k)
         if (pairs[k] < 0 || pairs[k] >= c->n_tracks) { acoss_set_error("pair index %d out of range", pairs[k]); return ACOSS_E_INVALID; }
@@ -728,6 +728,16 @@ int acoss_score_pairs_chen(acoss_ctx *c, const int32_t *pairs, int64_t K, const 
     CUDA_TRY(cudaMemcpyAsync(qmax_scores, c->scores.p, (size_t)K * 4, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaMemcpyAsync(dmax_scores, (float *)c->scores.p + K, (size_t)K * 4, cudaMemcpyDeviceToHost, c->stream));
     return acoss_sync(c);
+}
+
+int acoss_score_pairs_chen_device(acoss_ctx *c, const int32_t *pairs_dev, int64_t K, const acoss_params *p, float *qmax_dev,
+                                  float *dmax_dev) {
+    if (!c || (K > 0 && (!pairs_dev || !qmax_dev || !dmax_dev))) { acoss_set_error("score_pairs_chen_device: NULL argument"); return ACOSS_E_INVALID; }
+    TRY(check_params(c, p));
+    if (K <= 0) return ACOSS_OK;
+    acoss_params pp = *p;                                    // run_pairs keeps its own copy for the deferred fallback
+    pp.align = ACOSS_ALIGN_QMAX;
+    return run_pairs(c, pairs_dev, K, &pp, qmax_dev, nullptr, dmax_dev);
 }
 
 int acoss_oti_pairs(acoss_ctx *c, const int32_t *pairs, int64_t K, int32_t noti, int32_t *oti) {

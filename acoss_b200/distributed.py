@@ -144,10 +144,13 @@ def all_pairwise_distributed(alg, symmetric=True, score_fn=None, fill_on=None, c
     `alg.Ds[key]` holds the full (symmetrised) score matrix of every key (`fill_on=r`: only rank r's, the other
     ranks skip the assembly — what a benchmark run that evaluates on one rank wants).
 
-    Serra09-style plugins (one score per pair; `_pair_array`, `load_features`, `Ds`, `N`, `m`, `tau`) are
-    balanced by DP cells (n_q - m tau)(n_r - m tau).  Plugins with several scores per pair (EarlyFusion:
-    'mfccs', 'ssms', 'chromas', 'early') provide `pair_weights(pairs)` and `score_pairs(pairs) -> float32
-    (n_keys, n)` with rows in `alg.Ds` key order; their score rows travel in ONE gather.
+    Serra09-style plugins (`_pair_array`, `load_features`, `Ds`, `N`, `m`, `tau`) are balanced by DP cells
+    (n_q - m tau)(n_r - m tau) over the list-free triangle shard.  Those with several scores per pair (ChenFusion:
+    'qmax', 'dmax') provide `score_pairs(pairs)` and keep that shard.  Other plugins with several scores per pair
+    (EarlyFusion: 'mfccs', 'ssms', 'chromas', 'early') also provide `pair_weights(pairs)`.
+    Row contract: every scoring call returns float32 (len(alg.Ds), n) with rows in `alg.Ds` key order (a plugin
+    with one key may return (n,)); an empty shard contributes (rows, 0); a tile of any other shape is a scoring
+    failure.  All score rows travel in ONE gather.
     `score_fn(pairs)` overrides the scoring call (CPU tests).  The shard is scored in tiles of `alg.tile_pairs`;
     with `checkpoint_dir` every finished tile is saved per rank and an interrupted run resumes from the tiles it
     finds (same world size, pair list and tile size).  `timings` (a dict) receives the seconds of each phase."""
@@ -177,6 +180,16 @@ def all_pairwise_distributed(alg, symmetric=True, score_fn=None, fill_on=None, c
         mine = pairs[bounds[rank]:bounds[rank + 1]]
         n_pairs = len(pairs)
     keys = list(alg.Ds.keys())
+    rows = len(keys)
+
+    def tile_rows(got, n):                                  # the row contract: (rows, n); (n,) only for one key
+        got = np.asarray(got, dtype=np.float32)
+        if rows == 1 and got.ndim == 1:
+            got = got.reshape(1, -1)
+        if got.shape != (rows, n):
+            raise ValueError("a tile of %d pairs was scored as shape %r; the score types %r need (%d, %d)"
+                             % (n, got.shape, keys, rows, n))
+        return got
     tile = int(getattr(alg, "tile_pairs", 1 << 16))
     if score_fn is not None:
         score_tile = lambda p: np.asarray(score_fn(p), dtype=np.float32)
@@ -207,7 +220,7 @@ def all_pairwise_distributed(alg, symmetric=True, score_fn=None, fill_on=None, c
                     save(t, got)
             else:
                 resumed += 1
-            parts.append(got)
+            parts.append(tile_rows(got, len(p)))
     except Exception as e:                                  # noqa: BLE001 - reported to every rank below
         failure = e
     # A rank whose scoring failed must not leave the others waiting in the gather: agree on the outcome first (one
@@ -219,13 +232,10 @@ def all_pairwise_distributed(alg, symmetric=True, score_fn=None, fill_on=None, c
             raise RuntimeError("all_pairwise_distributed: scoring failed on another rank (rank %d had finished its shard)" % rank)
     if failure is not None:
         raise RuntimeError("all_pairwise_distributed: scoring failed on rank %d: %s" % (rank, failure)) from failure
-    local = np.concatenate(parts, axis=-1) if parts else np.zeros(0, np.float32)
+    local = np.concatenate(parts, axis=1) if parts else np.zeros((rows, 0), np.float32)
     t2 = time.perf_counter()
-    rows = 1 if local.ndim == 1 else local.shape[0]
-    if rows not in (1, len(keys)):
-        raise ValueError("score rows (%d) do not match the score types %r" % (rows, keys))
     # one gather for all score rows: rank r contributes rows x (bounds[r+1] - bounds[r]) floats, row-major
-    flat = np.ascontiguousarray(local.reshape(rows, -1)).ravel()
+    flat = np.ascontiguousarray(local).ravel()
     full = gather_scores(torch.from_numpy(flat).to(dev), bounds * rows, rank, world)
     if dev.type == "cuda":
         torch.cuda.synchronize(dev)

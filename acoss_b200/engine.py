@@ -161,6 +161,14 @@ class Engine:
         params = params or default_params()
         check(self._lib.acoss_score_pairs_device(self._ctx, pairs_ptr, int(n_pairs), C.byref(params), scores_ptr))
 
+    def score_pairs_chen_device(self, pairs_ptr: int, n_pairs: int, qmax_ptr: int, dmax_ptr: int,
+                                params: Params | None = None):
+        """ChenFusion flavour of score_pairs_device (acoss_score_pairs_chen_device): Qmax and Dmax of the same CRPs
+        into two device buffers, asynchronous on the engine stream; call sync()."""
+        params = params or default_params()
+        check(self._lib.acoss_score_pairs_chen_device(self._ctx, pairs_ptr, int(n_pairs), C.byref(params), qmax_ptr,
+                                                      dmax_ptr))
+
     def sync(self):
         check(self._lib.acoss_sync(self._ctx))
 

@@ -124,6 +124,13 @@ void *acoss_stream(acoss_ctx *ctx);
  * Ds["qmax"][i][j] / Ds["dmax"][i][j].  p->align is ignored.  Host buffers. */
 int acoss_score_pairs_chen(acoss_ctx *ctx, const int32_t *pairs, int64_t n_pairs, const acoss_params *p,
                            float *qmax_scores, float *dmax_scores);
+/* Same with DEVICE buffers (pairs, qmax_dev and dmax_dev in HBM), asynchronous on the context's stream like
+ * acoss_score_pairs_device: the call enqueues all its work and returns without a host synchronisation; acoss_sync()
+ * waits for it.  Flagged pairs are re-scored by the exact path for both alignments, inside the enqueued work up to
+ * 4 x 16 of them and the remainder inside acoss_sync(), so both outputs are complete after acoss_sync().  p->align is
+ * ignored.  Used for device-resident timing and for NCCL hand-off. */
+int acoss_score_pairs_chen_device(acoss_ctx *ctx, const int32_t *pairs_dev, int64_t n_pairs, const acoss_params *p,
+                                  float *qmax_dev, float *dmax_dev);
 
 /* K1 only — essentia optimalTranspositionIndex (inside ChromaCrossSimilarity, App. A1). */
 int acoss_oti_pairs(acoss_ctx *ctx, const int32_t *pairs, int64_t n_pairs, int32_t noti, int32_t *oti);
