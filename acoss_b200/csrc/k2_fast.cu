@@ -68,11 +68,12 @@ struct FastLayout {
     size_t slot_bytes;
     size_t off_hdr, off_rrot, off_aaf, off_bbf, off_aai, off_bbi, off_lo, off_w, off_cb, off_sh, off_cnt,
         off_cand, off_candz, off_zin, off_zout, off_rowpack, off_pool, off_pcnt, off_samp_r, off_samp_c,
-        off_lsel, off_wlist, off_wcnt, off_win, off_qpl, off_rpl, off_lsum, off_tcq;
+        off_lsel, off_wlist, off_wcnt, off_win, off_qpl, off_rpl, off_lsum, off_tcq, off_rq;
     int max_rows, max_cols, max_frames, lines, pool_cap;
     int plane_frames;                   // frames per byte plane of the tensor sweeps (zero padded past the track end)
     int slog;                           // log2 of the diagonal sampling stride S
     int nst_r, nst_c;                   // sample slots per row (ceil(max_cols / S)) / per column
+    int rq_pitch;                       // re-queue words per slot and orientation of the tensor histogram sweeps
 };
 
 __host__ __device__ inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
@@ -133,7 +134,11 @@ FastLayout make_layout(const SlotGeom &g, int max_frames) {
     L.off_qpl = take((size_t)3 * L.plane_frames * 16);          // query byte planes [h, l1, l2][frame][16]
     L.off_rpl = take((size_t)3 * L.plane_frames * 16);          // rotated reference byte planes
     L.off_lsum = take((size_t)2 * L.plane_frames * 4);          // per frame: sum of its h bytes | sum of its l1 bytes << 16 (q, r)
-    L.off_tcq = take(4 * 4);                                    // next work item of each tensor sweep (slot 0's copy serves the call)
+    // slot 0's copy serves the call: next work item of each tensor sweep (hist col, hist row, emit, -), then per histogram
+    // orientation the main items decided and the items re-queued for a second dense level (k2_tc.inl)
+    L.off_tcq = take(8 * 4);
+    L.rq_pitch = (std::max(g.max_rows, g.max_cols) + 127) / 128;
+    L.off_rq = take((size_t)2 * L.rq_pitch * 4);                 // the re-queue, slot r / strips holds entry r (both orientations)
     L.slot_bytes = align_up(o, 256);
     return L;
 }
@@ -250,7 +255,7 @@ __global__ void __launch_bounds__(256) fast_prep_kernel(TrackSet ts, const int32
     uint32_t *cnt = slot_ptr<uint32_t>(scratch, L, slot, L.off_cnt);
     for (int i = threadIdx.x; i < L.lines; i += blockDim.x) cnt[i] = 0u;
     if (threadIdx.x == 0) { *slot_ptr<uint32_t>(scratch, L, slot, L.off_pcnt) = 0u; *slot_ptr<uint32_t>(scratch, L, slot, L.off_wcnt) = 0u; }
-    if (threadIdx.x < 4) slot_ptr<uint32_t>(scratch, L, slot, L.off_tcq)[threadIdx.x] = 0u;
+    if (threadIdx.x < 8) slot_ptr<uint32_t>(scratch, L, slot, L.off_tcq)[threadIdx.x] = 0u;
     __syncthreads();
     float *aaf = slot_ptr<float>(scratch, L, slot, L.off_aaf), *bbf = slot_ptr<float>(scratch, L, slot, L.off_bbf);
     int32_t *aai = slot_ptr<int32_t>(scratch, L, slot, L.off_aai), *bbi = slot_ptr<int32_t>(scratch, L, slot, L.off_bbi);
@@ -682,16 +687,9 @@ struct Bracket {
     bool done, miss, bad;
 };
 
-template <int STRIDE>
-__device__ __forceinline__ Bracket split_bracket(const uint32_t *hp, int hs, uint32_t mask, int fk, int ck, int lo, int sh,
-                                                 int rlo, int rhi, int target) {
-    int cum = 0, b1 = -2, b2 = -2, cb1 = 0, cend = 0;          // the underflow bin counts every item below the bracket
-    for (int b = 0; b < NBIN + 2; ++b) {                      // b - 1 = bin of the bracket; -1 under, NBIN over
-        const int c = (int)((hp[b * STRIDE] >> hs) & mask);
-        if (b1 < -1 && cum + c > fk) { b1 = b - 1; cb1 = cum; }
-        if (b2 < -1 && cum + c > ck) { b2 = b - 1; cend = cum + c; }
-        cum += c;
-    }
+// the bracket from the bins that hold the fk-th and ck-th items (b1, b2: bin - 1, -1 under, NBIN over, < -1 not found),
+// the items below bin b1 (cb1) and those up to bin b2 (cend)
+__device__ __forceinline__ Bracket make_bracket(int b1, int b2, int cb1, int cend, int lo, int sh, int rlo, int rhi, int target) {
     Bracket r;
     r.bad = (b1 < -1 || b2 < -1);
     const long long nlo = (b1 < 0) ? (long long)rlo : (long long)lo + ((long long)b1 << sh);
@@ -704,6 +702,19 @@ __device__ __forceinline__ Bracket split_bracket(const uint32_t *hp, int hs, uin
     r.done = !r.miss && ((cend - cb1 <= target) || (sh == 0));
     r.lo = (int)nlo; r.w = (int)range; r.below = cb1; r.sh = sh2;
     return r;
+}
+
+template <int STRIDE>
+__device__ __forceinline__ Bracket split_bracket(const uint32_t *hp, int hs, uint32_t mask, int fk, int ck, int lo, int sh,
+                                                 int rlo, int rhi, int target) {
+    int cum = 0, b1 = -2, b2 = -2, cb1 = 0, cend = 0;          // the underflow bin counts every item below the bracket
+    for (int b = 0; b < NBIN + 2; ++b) {                      // b - 1 = bin of the bracket; -1 under, NBIN over
+        const int c = (int)((hp[b * STRIDE] >> hs) & mask);
+        if (b1 < -1 && cum + c > fk) { b1 = b - 1; cb1 = cum; }
+        if (b2 < -1 && cum + c > ck) { b2 = b - 1; cend = cum + c; }
+        cum += c;
+    }
+    return make_bracket(b1, b2, cb1, cend, lo, sh, rlo, rhi, target);
 }
 
 constexpr int SPARSE_LEVELS = 3;
@@ -1633,8 +1644,8 @@ int launch_k2_fast(const TrackSet &ts, const int32_t *pairs, const int32_t *oti,
         // tensor sweeps (k2_tc.inl): one CTA = 128 owned lines; items from tcgen05.mma.kind::i8 over the byte planes
         const int tstrips_c = (g.max_cols + 127) / 128, tstrips_r = (g.max_rows + 127) / 128;
         // (one CTA per SM: it holds all 512 TMEM columns; the requested shared memory keeps a second one off the SM)
-        const size_t smem_h = std::max(sizeof(TcSmem<TC_NP_HIST>) + (size_t)(NBIN + 2) * 128 * 4, (size_t)120 * 1024);
-        const size_t smem_e = std::max(sizeof(TcSmem<TC_NP_EMIT>) + (size_t)(TC_CONS / 32) * (TC_STAGE * 32 * 8 + 64), (size_t)120 * 1024);
+        const size_t smem_h = std::max(sizeof(TcHistSmem), (size_t)120 * 1024);
+        const size_t smem_e = std::max(sizeof(TcSmem<TC_NP_EMIT, TC_NB_EMIT>) + (size_t)(TC_CONS / 32) * (TC_STAGE * 32 * 8 + 64), (size_t)120 * 1024);
         static bool tc_attr_done[64] = {false};
         if (!tc_attr_done[dev & 63]) {
             CUDA_TRY(cudaFuncSetAttribute(tc_hist_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_h));
@@ -1646,7 +1657,8 @@ int launch_k2_fast(const TrackSet &ts, const int32_t *pairs, const int32_t *oti,
         static int tc_sms[64] = {0};
         if (!tc_sms[dev & 63]) CUDA_TRY(cudaDeviceGetAttribute(&tc_sms[dev & 63], cudaDevAttrMultiProcessorCount, dev));
         auto tc_grid = [&](int64_t items) { return (unsigned)std::min<int64_t>(items, tc_sms[dev & 63]); };
-        // one launch per orientation: an item that still holds DENSE2_MIN_LIVE live lines after its sweep is swept again at once
+        // one launch per orientation: an item that still holds DENSE2_MIN_LIVE live lines after its sweep is re-queued and swept
+        // again by the same CTAs once every item has had its first level
         tb(K2K_HIST_COL);
         tc_hist_kernel<0><<<tc_grid((int64_t)n * tstrips_c), TC_THREADS, smem_h, st>>>(ts, pairs, first, n, L, base, tstrips_c, sh3, status, dbg,
                                                                                        dbg + 12, glive, gcap);
